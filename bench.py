@@ -32,6 +32,9 @@ Other legs on the same line: `lm_ba` (configs[3], M2), `remerge` (§8f-1), `jlin
 
 --impl reference times the reference's own compiled sources (oracle/_ref; the restatement if missing) on bounded
 samples of the same scene and prints the best-CPU port beside it.
+
+--dump-outputs DIR writes what the timed path computed in its last step (dump_outputs) as DIR/<name>.npy; the scene is
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -141,8 +144,9 @@ def algorithmic_bytes(n_rows, n_nodes, n_views, n_cand, n_valid):
 
 
 def reference_impl():
-    """(constructor, kind): the reference's own compiled sources (oracle/_ref, built where /root/reference exists and
-    shipped as object code) when they load here, else the restatement with the reference's loop structure."""
+    """(constructor, kind): the reference's own compiled sources (oracle/_ref, built by build() where the reference's
+    sources are present and shipped as object code) when they load here, else the restatement with the reference's loop
+    structure."""
     from oracle import oracle as orc
     try:
         from oracle import ref
@@ -286,6 +290,40 @@ def run_reference(args, rank, world):
     print(json.dumps(line))
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(eng, out_dir, node_begin, node_end):
+    """What a caller of TriEngine.run() receives for the nodes [node_begin, node_end) (this rank's own source images),
+    as float64 .npy files: each node's record (best candidate's 3D line = start, end, two depths, uncertainty; its
+    score; its neighbour (image id, line id); candidate and valid-connection counts) and its valid connections (neighbour
+    image id, line id), sorted within each node because they form a set. `node_index` holds the scene-wide index of each
+    dumped node: all of them, or a fixed seeded sample of them when the whole would exceed DUMP_BUDGET_BYTES."""
+    nodes = eng.get_nodes()
+    off, edges = eng.get_all_valid_edges()
+    idx = np.arange(node_begin, node_end)
+    n_edges = int(off[node_end] - off[node_begin])
+    per_node, per_edge = 8 * 16, 8 * 2  # bytes per node (15 values, its index, its offset), per valid connection
+    total = per_node * len(idx) + per_edge * n_edges
+    if total > DUMP_BUDGET_BYTES:
+        k = int(0.9 * len(idx) * DUMP_BUDGET_BYTES / total)  # 10% margin: connection counts vary from node to node
+        idx = np.sort(np.random.default_rng(0).choice(idx, k, replace=False))
+    cnt = off[idx + 1] - off[idx]
+    starts = np.concatenate([[0], np.cumsum(cnt)])
+    rows = np.repeat(off[idx] - starts[:-1], cnt) + np.arange(int(starts[-1]))
+    node_of = np.repeat(np.arange(len(idx)), cnt)
+    e = edges[rows]
+    e = e[np.lexsort((e[:, 1], e[:, 0], node_of))]
+    nodes = nodes[idx]
+    arrays = {"node_index": idx, "node_line": nodes["line"], "node_score": nodes["score"],
+              "node_best_neighbor": np.stack([nodes["ng_view"], nodes["ng_line"]], 1),
+              "node_counts": np.stack([nodes["n_cand"], nodes["n_valid"]], 1),
+              "valid_edge_off": starts, "valid_edges": e}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float64))
+
+
 def bind_to_gpu_numa_node(local_rank):
     """One process per GPU: run on (and therefore allocate pinned host buffers from) the CPU cores next to this rank's
     GPU, so that N ranks uploading at once do not pull their pages across the socket interconnect. Best effort."""
@@ -321,6 +359,8 @@ def main():
     ap.add_argument("--value-groups", type=int, default=1,
                     help="pipeline groups of the device-resident leg (1: the node kernel runs alone and is timed cleanly for the "
                          "roofline; >1 hides the row preparation of group g+1 under the node kernel of group g)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step for rank 0's source images as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     rank = int(os.environ.get("RANK", 0))
@@ -419,6 +459,8 @@ def main():
     ms_total = e0.elapsed_time(e1)
     launches = eng.stats()["n_kernel_launches"] - launches0
     n_edges_total = gather.check() if gather is not None else None  # asserts the exchange did not overflow
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs, int(scene.line_off[per * rank]), int(scene.line_off[per * (rank + 1)]))
     ms_total = reduce_max(ms_total)
     rows_all = reduce_sum(n_rows_rank)
     value = rows_all * args.steps / (ms_total * 1e-3)
@@ -729,19 +771,22 @@ def side_legs(args, eng, rank, world, local_rank, barrier, reduce_max, reduce_su
     my_imgs = [imgs[i] for i in mine]
     det.detect_batch(my_imgs[:64], image_index=mine[:64])  # warm-up
     barrier()
+    kj_ms = []
     t0 = time.perf_counter()
-    if world == 1:
-        res = det.detect_batch(my_imgs, image_index=mine)
-        n_vps = sum(r.count_vps() for r in res)
-    else:
-        res = lmdist.detect_vps_sharded(det.detect_batch, imgs, rank, world)
-        n_vps = sum(len(v) for v in res[1])
+    for _ in range(args.steps):  # one step = every image once
+        if world == 1:
+            res = det.detect_batch(my_imgs, image_index=mine)
+            n_vps = sum(r.count_vps() for r in res)
+        else:
+            res = lmdist.detect_vps_sharded(det.detect_batch, imgs, rank, world)
+            n_vps = sum(len(v) for v in res[1])
+        kj_ms.append(det.stats()["kernel_ms"])  # kernel time of this rank's last detect_batch call
     torch.cuda.synchronize()
-    dt = reduce_max(time.perf_counter() - t0)
-    kj = reduce_max(det.stats()["kernel_ms"]) * 1e-3
+    dt = reduce_max(time.perf_counter() - t0) / args.steps
+    kj = reduce_max(float(np.mean(kj_ms))) * 1e-3
     kjl = km.get("jlinkage_kernel", {})
     b_j = 1000 * 300 * (16 + 4)  # per GPU: float4 segment in, label out
-    jl = {"metric": "J-Linkage images/sec", "unit": "images/s",
+    jl = {"metric": "J-Linkage images/sec", "unit": "images/s", "steps": args.steps,
           "config": {"workload": "rome16k-slice", "images": n_img, "segments_per_image": 300, "hypotheses": 5000,
                      "vps_found": int(n_vps),
                      "parallelism": "images dealt by segment count, labels + VPs all-gathered" if world > 1 else "1 GPU"},
@@ -788,7 +833,7 @@ def side_legs(args, eng, rank, world, local_rank, barrier, reduce_max, reduce_su
     e3.add_matches_bulk(*sc2.bulk_matches(ids3))
     e3.set_shard(vb, ve)
     g3 = lmdist.NodeGather(e3, world, rank, shards=shards) if world > 1 else None
-    nst = max(2, min(args.steps, 5))
+    nst = args.steps
     for _ in range(2):
         s3 = e3.run()
         if g3 is not None:

@@ -1,12 +1,12 @@
 """Runner-level drop-in (BASELINE.json configs[0]: the reference plumbing on a 10-image scene; SURVEY.md §8d config 1:
 V=10, L=800, N=9, K=10 through limap.runners.line_triangulation with load_det / load_match artefacts).
 
-  * CPU, where /root/reference exists: the REFERENCE'S OWN runner file, src/limap/runners/line_triangulation.py, is
-    loaded by path and executed UNMODIFIED against this repository's `limap` package (base, triangulation, merging,
-    optimize, vplib, util.io, runners, visualize). No GPU is needed because the three engine classes are replaced by
-    oracle-backed stand-ins for the duration of the test. Its result must equal the result of this repository's own
-    runner mirror (limap_b200/runners.py) on the same artefacts: same tracks, same refined lines, same files on
-    disk, same [Track Report].
+  * CPU: the REFERENCE'S OWN runner file, src/limap/runners/line_triangulation.py, loaded by path and executed
+    UNMODIFIED against this repository's `limap` package (base, triangulation, merging, optimize, vplib, util.io,
+    runners, visualize), with the three engine classes replaced by oracle-backed stand-ins. What it returned and wrote is
+    stored in tests/golden/ref/runner_line_triangulation.npz (recorded by tests/golden/make_ref_golden.py with
+    LIMAP_REFERENCE pointing at a LIMAP source tree). This repository's own runner mirror (limap_b200/runners.py) on the
+    same artefacts must reproduce it: same tracks, same refined lines, same files on disk, same [Track Report].
   * GPU: the runner mirror with the real CUDA engines against the same mirror on the oracle stand-ins: track
     membership bit-exact, refined endpoints 1e-4, [Track Report] equal.
 Together: reference runner == mirror (same surface), mirror on CUDA == mirror on the oracle (same arithmetic)."""
@@ -22,8 +22,14 @@ from limap_b200.config import default_runner_config
 from limap_b200.synth import CONFIGS, make_scene
 
 from runner_utils import imagecols_of, install_oracle_backend, summarize, write_artifacts
+from ref_golden import reference as _reference
 
-REF_RUNNER = "/root/reference/src/limap/runners/line_triangulation.py"
+RUNNER_FILES = ("image_list.txt", "metainfos.txt", "alltracks.txt", "finaltracks/track_0.txt", "triangulated_lines_nv4.obj")
+
+
+def _reference_tree_file(rel):
+    """A file of the LIMAP source tree at $LIMAP_REFERENCE (read only when recording the golden outputs)."""
+    return os.path.join(os.environ["LIMAP_REFERENCE"], rel)
 
 
 def _scene(small):
@@ -49,41 +55,50 @@ def _report(tracks):
     return vis.Open3DTrackVisualizer(tracks).track_report()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_RUNNER), reason="the reference tree is only present in the authoring container")
-def test_reference_runner_file_runs_unmodified_on_this_surface(tmp_path, monkeypatch, capsys):
+def _record_reference_runner(tmp_path, monkeypatch, capsys, sc, cfg):
     import copy
-    install_oracle_backend(monkeypatch)
     # the only names the reference runner imports that are not part of the hot path: pycolmap (logging) -- stubbed
     pyc = types.ModuleType("pycolmap")
     pyc.logging = types.SimpleNamespace(info=lambda *a, **k: None, warning=lambda *a, **k: None, error=lambda *a, **k: None)
     monkeypatch.setitem(sys.modules, "pycolmap", pyc)
     monkeypatch.setitem(sys.modules, "pycolmap.logging", pyc.logging)
     import limap  # noqa: F401  (alias package: limap.X -> limap_b200.X)
-    spec = importlib.util.spec_from_file_location("reference_line_triangulation", REF_RUNNER)
+    path = _reference_tree_file("src/limap/runners/line_triangulation.py")
+    spec = importlib.util.spec_from_file_location("reference_line_triangulation", path)
     ref_mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref_mod)
-    with open(REF_RUNNER) as f:
+    with open(path) as f:
         assert "def line_triangulation(cfg, imagecols, neighbors=None, ranges=None):" in f.read()
-
-    sc = _scene(small=True)
-    cfg = _cfg(tmp_path, sc)
     cfg_ref = copy.deepcopy(cfg)
     cfg_ref["output_dir"] = str(tmp_path / "out_ref")
     ref_tracks = ref_mod.line_triangulation(cfg_ref, imagecols_of(sc), neighbors=dict(sc.neighbors), ranges=sc.ranges)
-    out = capsys.readouterr().out
-    assert "[Track Report]" in out
+    assert "[Track Report]" in capsys.readouterr().out
+    members, lines = summarize(ref_tracks)
+    out = dict(track_off=np.concatenate([[0], np.cumsum([len(m) for m in members])]),
+               members=np.asarray([x for m in members for x in m], np.int32).reshape(-1, 2), lines=lines,
+               report=np.asarray(_report(ref_tracks)),
+               imagecols_npy=np.asarray((tmp_path / "out_ref" / "imagecols.npy").exists()))
+    for k, rel in enumerate(RUNNER_FILES):
+        out[f"file_{k}"] = np.frombuffer((tmp_path / "out_ref" / rel).read_bytes(), np.uint8)
+    return out
+
+
+def test_reference_runner_file_runs_unmodified_on_this_surface(tmp_path, monkeypatch, capsys):
+    install_oracle_backend(monkeypatch)
+    sc = _scene(small=True)
+    cfg = _cfg(tmp_path, sc)
+    r = _reference("runner_line_triangulation", lambda: _record_reference_runner(tmp_path, monkeypatch, capsys, sc, cfg))
     my_tracks = _run_mirror(cfg, sc)
-    (m_ref, l_ref), (m_my, l_my) = summarize(ref_tracks), summarize(my_tracks)
+    m_my, l_my = summarize(my_tracks)
+    off = r["track_off"]
+    m_ref = [tuple(map(tuple, r["members"][off[k]:off[k + 1]].tolist())) for k in range(len(off) - 1)]
     assert len(m_ref) > 20 and m_ref == m_my
-    assert np.array_equal(l_ref, l_my)  # same backend, same call sequence: bit-identical
-    assert _report(ref_tracks) == _report(my_tracks)
+    assert np.array_equal(r["lines"], l_my)  # same backend, same call sequence: bit-identical
+    assert tuple(r["report"].tolist()) == _report(my_tracks)
     # the files a user finds afterwards
-    for rel in ("image_list.txt", "imagecols.npy", "metainfos.txt", "alltracks.txt", "finaltracks/track_0.txt",
-                "triangulated_lines_nv4.obj"):
-        a, b = tmp_path / "out_ref" / rel, tmp_path / "out" / rel
-        assert a.exists() and b.exists(), rel
-        if rel.endswith(".txt") or rel.endswith(".obj"):
-            assert a.read_text() == b.read_text(), rel
+    assert bool(r["imagecols_npy"]) and (tmp_path / "out" / "imagecols.npy").exists()
+    for k, rel in enumerate(RUNNER_FILES):
+        assert (tmp_path / "out" / rel).read_bytes() == r[f"file_{k}"].tobytes(), rel
     import limap.util.io as limapio
     back, cfg_back, ic_back, segs_back = limapio.read_folder_linetracks_with_info(str(tmp_path / "out" / "finaltracks"))
     assert len(back) == len(my_tracks) and ic_back.NumImages() == len(sc.img_ids) and len(segs_back) == len(sc.img_ids)
@@ -107,22 +122,41 @@ def test_runner_mirror_cuda_equals_oracle_backend_hypersim10(tmp_path, monkeypat
     assert (tmp_path / "out" / "finaltracks" / "track_0.txt").exists()
 
 
-REF_TEST_LINEBASE = "/root/reference/tests/base/test_linebase.py"
+def _record_reference_linebase_test():
+    """The one test of the reference's own suite that touches a hot-path type (tests/base/test_linebase.py::test_line2d),
+    run unmodified against `import limap` = this repository's alias package, with Line2d recording what it is asked and
+    numpy.testing recording what is compared: the known-answer vectors of that test."""
+    import numpy.testing as npt
+    import limap
+    made, checks = [], []
+    line2d = limap.base.Line2d
 
+    def recording_line2d(start, end):
+        made.append(np.concatenate([np.asarray(start, float), np.asarray(end, float)]))
+        return line2d(start, end)
 
-@pytest.mark.skipif(not os.path.exists(REF_TEST_LINEBASE), reason="the reference tree is only present in the authoring container")
-def test_reference_own_linebase_test_passes_on_the_mirror():
-    """The one test of the reference's own suite that touches a hot-path type (tests/base/test_linebase.py), loaded by
-    path and run unmodified against `import limap` = this repository's alias package."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_test_linebase", REF_TEST_LINEBASE)
+    def recording_allclose(actual, desired, rtol=1e-7, atol=0):
+        checks.append((np.atleast_1d(np.asarray(desired, float)), rtol, atol))
+        npt.assert_allclose(actual, desired, rtol=rtol, atol=atol)
+    spec = importlib.util.spec_from_file_location("ref_test_linebase", _reference_tree_file("tests/base/test_linebase.py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
-    import limap
     assert mod.limap is limap and limap.base.__name__ == "limap_b200.base"
-    ran = 0
-    for name in dir(mod):
-        if name.startswith("test_"):
-            getattr(mod, name)()
-            ran += 1
-    assert ran >= 1
+    mod.limap = types.SimpleNamespace(base=types.SimpleNamespace(Line2d=recording_line2d))
+    mod.npt = types.SimpleNamespace(assert_allclose=recording_allclose)
+    mod.test_line2d()
+    assert len(made) == 1 and len(checks) == 2
+    return dict(line=made[0], length=checks[0][0], direction=checks[1][0],
+                tol=np.array([[c[1], c[2]] for c in checks]))
+
+
+def test_reference_own_linebase_test_passes_on_the_mirror():
+    """tests/base/test_linebase.py::test_line2d of the reference's own suite on the mirror: Line2d((0, 0), (1, 1)) has
+    length sqrt(2) and direction (1, 1) / sqrt(2), with that test's tolerances (tests/golden/ref/linebase_test_line2d.npz)."""
+    import numpy.testing as npt
+    import limap
+    assert limap.base.__name__ == "limap_b200.base"
+    r = _reference("linebase_test_line2d", _record_reference_linebase_test)
+    line = limap.base.Line2d(r["line"][:2], r["line"][2:])
+    npt.assert_allclose(line.length(), r["length"][0], rtol=r["tol"][0, 0], atol=r["tol"][0, 1])
+    npt.assert_allclose(line.direction(), r["direction"], rtol=r["tol"][1, 0], atol=r["tol"][1, 1])
