@@ -148,6 +148,7 @@ struct lm_ctx {
   int gather_world = 0;
   bool edges_count_on_device = false; // n_edges_dev is still on the device (lm_tri_unpack_messages)
   int cap_hint = 0;                  // staging capacity of the node kernel, from the previous run (0: default)
+  int cap_hint_cand = 0;             // the same for the split scorer: largest candidate count of a node (0: unknown)
   bool outside_shard_clean = false;  // node records / row offsets outside the shard were zero-filled
   int run_retry = 0;
   int sm_count = 148;
@@ -184,7 +185,7 @@ struct lm_ctx {
   DevBuf d_blk_row_off, d_blk_src, d_blk_ng, d_blk_pair_off;
   DevBuf d_key, d_key2, d_val, d_val2, d_sort_tmp;
   DevBuf d_node_row_off, d_scalars; // scalars: [0] max_rows(uint) [1] err(int) ; counters at +16
-  DevBuf d_nodes, d_row_state, d_row_cand, d_slab;
+  DevBuf d_nodes, d_row_state, d_row_cand, d_slab, d_cand;
   DevBuf d_edges, d_edges2, d_edge_keys, d_edge_keys2, d_edge_w, d_edge_cnt;
   DevBuf d_g_flag, d_g_pos, d_g_kc, d_g_wc, d_g_occ, d_g_occ2, d_g_hk, d_g_hk2, d_g_gidx, d_g_gnode, d_g_k1, d_g_k1b, d_g_k2, d_g_k2b;
   DevBuf d_nvalid, d_edge_off, d_edge_ng; // compact valid_edges_ of the shard (node-major, candidate order)
@@ -330,7 +331,7 @@ void lm_ctx_destroy(lm_ctx *c) {
   DevBuf *bufs[] = {&c->d_scan_tmp, &c->d_local_off, &c->d_segs_raw, &c->d_img_ids, &c->d_host_edges, &c->d_views, &c->d_segs, &c->d_node_view, &c->d_line_off, &c->d_pairs, &c->d_blk_row_off,
                     &c->d_blk_src, &c->d_blk_ng, &c->d_blk_pair_off, &c->d_key, &c->d_key2, &c->d_val, &c->d_val2,
                     &c->d_sort_tmp, &c->d_node_row_off, &c->d_scalars, &c->d_nodes, &c->d_row_state, &c->d_row_cand,
-                    &c->d_slab, &c->d_edges, &c->d_edges2, &c->d_edge_keys, &c->d_edge_keys2, &c->d_edge_w,
+                    &c->d_slab, &c->d_cand, &c->d_edges, &c->d_edges2, &c->d_edge_keys, &c->d_edge_keys2, &c->d_edge_w,
                     &c->d_edge_cnt, &c->d_nvalid, &c->d_edge_off, &c->d_edge_ng, &c->d_ba_in, &c->d_ba_blocks, &c->d_ba_out, &c->d_raw_blocks, &c->d_bkey, &c->d_bkey2, &c->d_bval, &c->d_bval2, &c->d_blk_rows, &c->d_vp_label, &c->d_vp_voff, &c->d_vp_vps, &c->d_vp_pts, &c->d_vp_off, &c->d_vp_labels, &c->d_vp_nc, &c->d_vp_ps, &c->d_vp_mat, &c->d_mg_in, &c->d_mg_out, &c->d_mg_edges, &c->d_gather, &c->d_vp_idx, &c->d_sfm_in, &c->d_sfm_keys, &c->d_sfm_keys2, &c->d_sfm_a, &c->d_sfm_b, &c->d_sfm_c, &c->d_sfm_d, &c->d_g_flag, &c->d_g_pos, &c->d_g_kc, &c->d_g_wc, &c->d_g_occ, &c->d_g_occ2, &c->d_g_hk, &c->d_g_hk2, &c->d_g_gidx, &c->d_g_gnode, &c->d_g_k1, &c->d_g_k1b, &c->d_g_k2, &c->d_g_k2b};
   for (DevBuf *b : bufs) b->release();
   if (c->ev0) cudaEventDestroy(c->ev0);
@@ -857,7 +858,8 @@ int lm_tri_run(lm_ctx *c) {
     CU(cub::DeviceScan::ExclusiveSum(c->d_sort_tmp.p, tmps, c->d_blk_rows.as<int64_t>(), c->d_blk_row_off.as<int64_t>(),
                                      nb + 1, sp));
   }
-  // d_scalars words: [1] index error, [2] staging overflow, bytes 16..47 counters, words [16 + g] largest node of group g
+  // d_scalars words: [1] index error, [2] staging overflow, [3] largest candidate count of a node (split path), bytes
+  // 16..47 counters, words [16 + g] largest node of group g
   int *d_err = c->d_scalars.as<int>() + 1;
   unsigned long long *d_counters = reinterpret_cast<unsigned long long *>(c->d_scalars.as<char>() + 16);
   int launches = 0;
@@ -873,6 +875,7 @@ int lm_tri_run(lm_ctx *c) {
   p.row_cand = c->cfg.debug_mode ? c->d_row_cand.as<double>() : nullptr;
   p.counters = d_counters;
   p.overflow = c->d_scalars.as<int>() + 2;
+  p.max_cand = c->d_scalars.as<unsigned int>() + 3;
   p.node_begin = c->node_begin;
   p.node_end = c->node_end;
   const lm_tri_config &g = c->cfg;
@@ -965,6 +968,36 @@ int lm_tri_run(lm_ctx *c) {
     CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     c->evp.push_back(e);
   }
+  // Split form of the fast path (tri_gen_kernel + tri_score_kernel, the default): its staging capacity comes from the
+  // largest candidate count of a node, which the score kernel reports; LIMAP_B200_TRI_FUSED=1 (read per run) selects the
+  // fused tri_node_kernel. Exhaustive matching and the generic forms always run fused.
+  const int cap_split = c->cap_hint_cand > 0 ? c->cap_hint_cand : cap;
+  const bool split = fast_kernel && !exhaustive && !getenv("LIMAP_B200_TRI_FUSED") &&
+                     lm::tri_score_smem_bytes(cap_split) <= smem_limit;
+  // blocks [gb[g], gb[g + 1]) with whole source images form group g
+  std::vector<int> gb(n_groups + 1, nb);
+  gb[0] = 0;
+  int64_t max_group_rows = 0;
+  for (int g = 0; g < n_groups; ++g) {
+    int bg1 = nb;
+    if (g + 1 < n_groups) {
+      // small groups at both ends (smoothstep): the first one is the only one whose matches nothing else can hide, the
+      // last one is the only one whose results nothing else can hide
+      const double tg = (g + 1.0) / n_groups;
+      const int64_t target = (int64_t)((double)n_rows * (tg * tg * (3.0 - 2.0 * tg)));
+      bg1 = gb[g];
+      while (bg1 < nb && row_off[bg1] < target) ++bg1;
+      while (bg1 < nb && bg1 > 0 && blk[bg1].src_view == blk[bg1 - 1].src_view) ++bg1; // finish the image
+    }
+    gb[g + 1] = bg1;
+    max_group_rows = std::max(max_group_rows, row_off[bg1] - row_off[gb[g]]);
+  }
+  if (split) {
+    p.row_node = c->sorted_key;
+    p.cand_stride = std::max<int64_t>(max_group_rows * ns, 1);
+    CU(c->d_cand.ensure(sizeof(double) * lm::kCandFields * p.cand_stride));
+    p.cand = c->d_cand.as<double>();
+  }
   std::vector<int> group_has_kernel(n_groups, 0);
   CU(c->d_nvalid.ensure(4 * (n_shard_nodes + 2)));
   CU(c->d_local_off.ensure(4 * (n_shard_nodes + 2)));
@@ -972,17 +1005,8 @@ int lm_tri_run(lm_ctx *c) {
   CU(c->d_edge_ng.ensure(4 * std::max<int64_t>(n_rows * ns, 1)));
   for (int g = 0; g < n_groups; ++g) {
     // blocks [bg0, bg1) with whole source images, views [gv0, gv1)
-    int bg1 = nb, gv1 = ve;
-    if (g + 1 < n_groups) {
-      // small groups at both ends (smoothstep): the first one is the only one whose matches nothing else can hide, the
-      // last one is the only one whose results nothing else can hide
-      const double tg = (g + 1.0) / n_groups;
-      const int64_t target = (int64_t)((double)n_rows * (tg * tg * (3.0 - 2.0 * tg)));
-      bg1 = bg0;
-      while (bg1 < nb && row_off[bg1] < target) ++bg1;
-      while (bg1 < nb && bg1 > 0 && blk[bg1].src_view == blk[bg1 - 1].src_view) ++bg1; // finish the image
-      gv1 = (bg1 < nb) ? blk[bg1].src_view : ve;
-    }
+    const int bg1 = gb[g + 1];
+    const int gv1 = (g + 1 < n_groups && bg1 < nb) ? blk[bg1].src_view : ve;
     const int64_t rb = row_off[bg0], re = row_off[bg1];
     const int64_t node_lo = c->line_off[gv0], node_hi = c->line_off[gv1];
     if (!exhaustive && re > rb) {
@@ -1024,9 +1048,15 @@ int lm_tri_run(lm_ctx *c) {
     p.node_begin = node_lo;
     p.node_end = node_hi;
     const int64_t n_group_nodes = node_hi - node_lo;
-    size_t smem = lm::tri_smem_bytes(cap, fast_kernel);
+    size_t smem = split ? lm::tri_score_smem_bytes(cap_split) : lm::tri_smem_bytes(cap, fast_kernel);
     int grid;
-    if (smem <= smem_limit) {
+    if (split) {
+      p.use_slab = 0;
+      p.cap = cap_split;
+      p.row_begin = rb;
+      p.row_end = re;
+      grid = (int)std::min<int64_t>(n_group_nodes, (int64_t)1 << 30);
+    } else if (smem <= smem_limit) {
       p.use_slab = 0;
       p.cap = cap;
       grid = (int)std::min<int64_t>(n_group_nodes, (int64_t)1 << 30);
@@ -1041,11 +1071,12 @@ int lm_tri_run(lm_ctx *c) {
       smem = 0;
     }
     if (n_group_nodes > 0) {
-      CU(cudaEventRecord(c->evk[2 * g], s));
-      CU(lm::launch_tri_node_kernel(p, grid, 128, smem, s));
+      CU(cudaEventRecord(c->evk[2 * g], s)); // node kernel time: generation through scoring
+      if (split) CU(lm::launch_tri_split(p, grid, smem, s));
+      else CU(lm::launch_tri_node_kernel(p, grid, 128, smem, s));
       CU(cudaEventRecord(c->evk[2 * g + 1], s));
       group_has_kernel[g] = 1;
-      ++launches;
+      launches += split ? 2 : 1;
       // valid_edges_ of the group in compact form: per-node counts -> exclusive scan -> ordered scatter at the global
       // offsets
       {
@@ -1100,6 +1131,11 @@ int lm_tri_run(lm_ctx *c) {
   int need_cap = 32;
   while (need_cap < max_rows_all * ns) need_cap += 32;
   c->cap_hint = need_cap;
+  if (split) { // largest candidate count of a node in this run: the split scorer's capacity from now on
+    int need_cand = 32;
+    while (need_cand < (int)hs[3]) need_cand += 32;
+    c->cap_hint_cand = need_cand;
+  }
   if (hs[2] != 0) { // some node did not fit the staging area sized from the hint: repeat with the exact size
     if (c->run_retry) { c->run_retry = 0; return fail(LM_ERR_STATE, "node staging overflow after resizing"); }
     c->run_retry = 1;

@@ -50,6 +50,9 @@ size_t tri_smem_bytes(int cap, bool fast) {
   if (fast) return (size_t)cap * (20 * 8 + kWarps * 8 + 32 + 8 + 4 + 2 + kWarps * 2);
   return (size_t)cap * kCandBytes + (size_t)kWarps * 2 * (cap + kListExtra) * 4 + (size_t)kWarps * cap * 2;
 }
+// Split scorer (tri_score_kernel): the fast layout without the four segment coordinates (a 4-byte global segment index
+// instead) and without zs / ze / unc (read from the candidate records where phase C outputs them): 194 bytes per slot.
+size_t tri_score_smem_bytes(int cap) { return (size_t)cap * (13 * 8 + kWarps * 8 + 32 + 12 + 4 + 2 + kWarps * 2); }
 
 // fp32 copy of a candidate for the pruning gates (three 16-byte loads, conflict-free at 48-byte stride):
 // unit direction, endpoints relative to the source camera centre, squared scale-invariance limits of the
@@ -83,7 +86,9 @@ struct Slab {
   uint16_t *sidx;            // [cap] candidate of each sorted position
   double *psc;               // [kWarps][cap] scores of a warp's pair list
   uint16_t *pent;            // [kWarps][cap] j of a warp's pair list (rows contiguous)
+  uint32_t *seg;             // split layout only: [cap] global segment index (into TriParams::segs) of the candidate
   LM_D void carve(char *base, int cap, bool fast) {
+    seg = nullptr;
     if (fast) { carve_fast(base, cap); return; }
     gatef = nullptr; slam = nullptr; sidx = nullptr; psc = nullptr; pent = nullptr;
     double *d = reinterpret_cast<double *>(base);
@@ -112,6 +117,23 @@ struct Slab {
     slam = reinterpret_cast<float *>(row + cap);                  // byte 232 cap
     sidx = reinterpret_cast<uint16_t *>(slam + cap);              // byte 236 cap
     pent = sidx + cap;                                            // byte 238 cap, [kWarps][cap]
+    gate = nullptr; list = nullptr; list0 = nullptr; seg = nullptr;
+  }
+  // tri_score_kernel: tri_score_smem_bytes() per slot, no zs / ze / unc / q0..q3
+  LM_D void carve_split(char *base, int cap) {
+    double *d = reinterpret_cast<double *>(base);
+    sx = d; sy = sx + cap; sz = sy + cap; ex = sz + cap; ey = ex + cap; ez = ey + cap;
+    dx = ez + cap; dy = dx + cap; dz = dy + cap; score = dz + cap;
+    izs2 = score + cap; ize2 = izs2 + cap; inb = ize2 + cap;
+    psc = inb + cap;                                              // byte 104 cap
+    gatef = reinterpret_cast<GateRecF *>(psc + (size_t)kWarps * cap); // byte 136 cap (cap is a multiple of 32)
+    ng = reinterpret_cast<uint32_t *>(gatef + cap);               // byte 168 cap
+    row = ng + cap;
+    seg = row + cap;
+    slam = reinterpret_cast<float *>(seg + cap);                  // byte 180 cap
+    sidx = reinterpret_cast<uint16_t *>(slam + cap);              // byte 184 cap
+    pent = sidx + cap;                                            // byte 186 cap, [kWarps][cap]
+    zs = ze = unc = q0 = q1 = q2 = q3 = nullptr;
     gate = nullptr; list = nullptr; list0 = nullptr;
   }
 };
@@ -457,6 +479,7 @@ LM_D double angle2_deg(double t, double abs_cos) {
 // == exp(-max (v/sigma)^2 / 2), so the squared normalised deviations are maximised and one exponential is taken;
 // angles come from sin^2 (cross products) through the asin^2 series, distances stay squared, and the divisors
 // that depend on one candidate only (depths of l_i, |q_j|^2) are reciprocals prepared in phase A.
+template <bool SPLIT = false>
 LM_D double pair_score_fast(const TriParams &p, const Slab &sl, int i, int j, uint32_t vj) {
   const double EPS = consts<double>::eps();
   const LinkerDev<double> &c3 = p.l3d;
@@ -483,7 +506,15 @@ LM_D double pair_score_fast(const TriParams &p, const Slab &sl, int i, int j, ui
   const vec3<double> hs = proj_h(v.P, si), he = proj_h(v.P, ei);
   const double ws = 1.0 / (hs.z + EPS), we = 1.0 / (he.z + EPS);
   const vec2<double> as = mk2(hs.x * ws, hs.y * ws), ae = mk2(he.x * we, he.y * we);
-  const vec2<double> bs = mk2(sl.q0[j], sl.q1[j]), be = mk2(sl.q2[j], sl.q3[j]);
+  vec2<double> bs, be;
+  if constexpr (SPLIT) { // the split scorer keeps the global segment index of a candidate instead of its four coordinates
+    const double4 q = ld_seg(&p.segs[sl.seg[j]]);
+    bs = mk2(q.x, q.y);
+    be = mk2(q.z, q.w);
+  } else {
+    bs = mk2(sl.q0[j], sl.q1[j]);
+    be = mk2(sl.q2[j], sl.q3[j]);
+  }
   const vec2<double> va = ae - as, vb = be - bs;
   const double na2 = dot(va, va), nb2 = dot(vb, vb);
   const double dab = dot(va, vb);
@@ -601,6 +632,294 @@ LM_D bool gate2d(const TriParams &p, const seg<vec3<double>> &Li, const Slab &sl
     if (m > p.th_perp2_2d * (1.0 + REL) + REL) return false;
   }
   return true;
+}
+
+// ---- phases shared by the fused kernel and the split generate / score kernels ---------------------------------------
+// Staging of one candidate in the scorer's shared-memory layout: the direction, the three reciprocals of the reduced-form
+// scorer and the fp32 gate record (FAST) or the generic gate copy. SPLIT keeps the global segment index `segi` instead
+// of the segment coordinates and leaves zs / ze / unc in the candidate record.
+template <bool FAST, bool SPLIT>
+LM_D void stage_cand(const TriParams &p, const Slab &sl, int idx, const Cand &c, double4 l2, uint32_t ng, uint32_t row,
+                     vec3<double> C1, uint32_t segi = 0) {
+  const vec3<double> dr = c.e - c.s;
+  const double dn2 = dot(dr, dr);
+  const vec3<double> d = (dn2 > 0.0) ? dr * (1.0 / sqrt(dn2)) : dr;
+  sl.sx[idx] = c.s.x; sl.sy[idx] = c.s.y; sl.sz[idx] = c.s.z;
+  sl.ex[idx] = c.e.x; sl.ey[idx] = c.e.y; sl.ez[idx] = c.e.z;
+  sl.dx[idx] = d.x; sl.dy[idx] = d.y; sl.dz[idx] = d.z;
+  if constexpr (SPLIT) {
+    sl.seg[idx] = segi; // zs / ze / unc stay in the candidate record
+  } else {
+    sl.zs[idx] = c.zs; sl.ze[idx] = c.ze; sl.unc[idx] = c.unc;
+    sl.q0[idx] = l2.x; sl.q1[idx] = l2.y; sl.q2[idx] = l2.z; sl.q3[idx] = l2.w;
+  }
+  if (FAST) {
+    const double zs1 = c.zs + consts<double>::eps(), ze1 = c.ze + consts<double>::eps();
+    const double qx = l2.z - l2.x, qy = l2.w - l2.y;
+    sl.izs2[idx] = 1.0 / (zs1 * zs1); sl.ize2[idx] = 1.0 / (ze1 * ze1); sl.inb[idx] = 1.0 / (qx * qx + qy * qy);
+  }
+  sl.ng[idx] = ng;
+  sl.row[idx] = row;
+  if (FAST) {
+    // fp32 gate record: the endpoints as distances along the two source rays. Limits: th * (z + EPS) widened by
+    // 0.5% plus 1e-5 of the larger distance (fp32 rounding of the two lambdas and of their difference is below
+    // 2e-7 of it, |X_i - X_j| and |lambda_i - lambda_j| agree to 1e-15); see DESIGN.md "gates"
+    const double rad = fmax(fabs(c.lam_s), fabs(c.lam_e));
+    const double ls = p.l3d.th_scaleinv * (c.zs + consts<double>::eps()) * 1.005 + 1e-5 * rad;
+    const double le = p.l3d.th_scaleinv * (c.ze + consts<double>::eps()) * 1.005 + 1e-5 * rad;
+    GateRecF g;
+    g.dx = (float)d.x; g.dy = (float)d.y; g.dz = (float)d.z; g.lam_e = (float)c.lam_e;
+    g.lam_s = (float)c.lam_s; g.lim_s = (float)(ls * 1.000001); g.lim_e = (float)(le * 1.000001);
+    g.img = (int)(ng >> 16);
+    sl.gatef[idx] = g;
+    reinterpret_cast<float *>(sl.psc)[idx] = g.lam_s; // unsorted keys of the depth sort (scratch: the score lists)
+  } else {
+    // fp32 gate copy, relative to the source camera centre (keeps |coord| ~ depth)
+    const vec3<double> rs = c.s - C1, re = c.e - C1;
+    // scale-invariance limit th * (z + EPS) widened by 0.5% plus 1e-5 of the coordinate magnitude
+    // (fp32 rounding of the two endpoints is < 1e-6 of it); see DESIGN.md "gates"
+    const double rad = sqrt(fmax(dot(rs, rs), dot(re, re)));
+    const double ls = p.l3d.th_scaleinv * (c.zs + consts<double>::eps()) * 1.005 + 1e-5 * rad;
+    const double le = p.l3d.th_scaleinv * (c.ze + consts<double>::eps()) * 1.005 + 1e-5 * rad;
+    GateRec g;
+    g.dx = (float)d.x; g.dy = (float)d.y; g.dz = (float)d.z; g.lims2 = (float)(ls * ls * 1.000001);
+    g.sx = (float)rs.x; g.sy = (float)rs.y; g.sz = (float)rs.z; g.lime2 = (float)(le * le * 1.000001);
+    g.ex = (float)re.x; g.ey = (float)re.y; g.ez = (float)re.z;
+    g.pad = 0.f;
+    sl.gate[idx] = g;
+  }
+}
+
+// Candidate records of the split path: field-major, field f of slot q at cand[f * cand_stride + q] with q = (row -
+// row_begin) * NS + k. Fields (kCandFields in tri_kernels.cuh): sx sy sz ex ey ez zs ze unc lam_s lam_e.
+// zs / ze / unc (fields 6..8) of staged candidate i: from shared memory (fused) or from its record (split)
+template <bool SPLIT>
+LM_D double cand_field(const TriParams &p, const Slab &sl, const double *smem_field, int f, int i, int64_t slot0) {
+  if constexpr (SPLIT) return p.cand[f * p.cand_stride + slot0 + sl.row[i]];
+  else return smem_field[i];
+}
+
+// Phase B of the fast path: all-pairs scoring of the C staged candidates of a node into sl.score.
+template <bool SPLIT>
+LM_D void phase_b_fast(const TriParams &p, const Slab &sl, const int C, unsigned long long &n1_total,
+                       unsigned long long &n2_total) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const unsigned lt_mask = (1u << lane) - 1u;
+  const unsigned FULL = 0xffffffffu;
+  {
+    float *ltmp = reinterpret_cast<float *>(sl.psc);
+    const int C4 = (C + 3) & ~3;
+    if (tid < C4 - C) ltmp[C + tid] = __int_as_float(0x7f800000); // +inf pads: never below a key, never tie-winners
+    __syncthreads();
+    for (int i = tid; i < C; i += kThreads) {
+      const float li = ltmp[i];
+      int r = 0;
+      for (int j4 = 0; j4 < C4; j4 += 4) {
+        const float4 v = *reinterpret_cast<const float4 *>(ltmp + j4);
+        r += (v.x < li) || (v.x == li && j4 < i);
+        r += (v.y < li) || (v.y == li && j4 + 1 < i);
+        r += (v.z < li) || (v.z == li && j4 + 2 < i);
+        r += (v.w < li) || (v.w == li && j4 + 3 < i);
+      }
+      sl.slam[r] = li;
+      sl.sidx[r] = (uint16_t)i;
+    }
+    __syncthreads(); // ltmp (= the score lists) is dead from here on
+  }
+  const float *slam = sl.slam;
+  const uint16_t *sidx = sl.sidx;
+  double *psc = sl.psc + (size_t)warp * p.cap;
+  uint16_t *pent = sl.pent + (size_t)warp * p.cap;
+  // rows are dealt to the warps in equal shares (C = 100: 25 rows per warp, not 32 + 32 + 32 + 4), so the warps
+  // reach the barrier before phase C together
+  const int n_pass = (C + 32 * kWarps - 1) / (32 * kWarps);
+  const int G = (C + kWarps * n_pass - 1) / (kWarps * n_pass); // rows per warp and pass, <= 32
+  for (int pass = 0; pass < n_pass; ++pass) {
+    const int g0 = (pass * kWarps + warp) * G;
+    if (g0 >= C) break;
+    const int Gact = min(G, C - g0);
+    // B-window, lane = row: two binary searches over the sorted start distances
+    int lo = 0, W = 0;
+    if (lane < Gact) {
+      const float4 a1 = *reinterpret_cast<const float4 *>(&sl.gatef[g0 + lane].lam_s);
+      int hi = C;
+      if (a1.y < 3e37f) { // (false for inf / NaN limits: the whole node is the window then)
+        const float wa = a1.x - a1.y, wb = a1.x + a1.y;
+        int l = 0, h = C;
+        while (l < h) { const int m = (l + h) >> 1; if (slam[m] < wa) l = m + 1; else h = m; }
+        lo = l;
+        h = C;
+        while (l < h) { const int m = (l + h) >> 1; if (!(slam[m] > wb)) l = m + 1; else h = m; }
+        hi = l;
+      }
+      W = hi - lo;
+    }
+    int rr = 0;
+    while (rr < Gact) {
+      // B-gate, one row at a time, lane = window position: the other fp32 gates (end-point interval, angle, other
+      // image). The partners of a row are written in ascending candidate order (= ascending neighbour image:
+      // candidates are generated image by image) at the running fill of the warp's pair list; lane r keeps the
+      // offset and the count of row r of the chunk. A chunk ends when the next row would not fit the list.
+      const int cb = rr;
+      int fill = 0, off = 0, n = 0;
+      for (; rr < Gact; ++rr) {
+        const int lo_r = __shfl_sync(FULL, lo, rr), W_r = __shfl_sync(FULL, W, rr);
+        const float4 a0 = *reinterpret_cast<const float4 *>(&sl.gatef[g0 + rr].dx);
+        const float4 a1 = *reinterpret_cast<const float4 *>(&sl.gatef[g0 + rr].lam_s);
+        int n_r = 0;
+        if (W_r <= 32) {
+          int j = 0x7fffffff;
+          bool ok = false;
+          if (lane < W_r) {
+            j = sidx[lo_r + lane];
+            const float4 gj = *reinterpret_cast<const float4 *>(&sl.gatef[j].dx);
+            const int imgj = sl.gatef[j].img;
+            ok = (imgj != __float_as_int(a1.w)) && !(fabsf(gj.w - a0.w) > a1.z) &&
+                 !(fabsf(a0.x * gj.x + a0.y * gj.y + a0.z * gj.z) < p.cos_th3d_f);
+          }
+          unsigned m = __ballot_sync(FULL, ok);
+          n_r = __popc(m);
+          if (n_r) {
+            if (fill + n_r > p.cap) break; // (a row has fewer than C <= cap partners: an empty list always takes it)
+            int rank = 0;
+            while (m) { // rank among the partners by candidate index: n_r independent shuffles
+              const int t = __ffs((int)m) - 1;
+              m &= m - 1;
+              rank += __shfl_sync(FULL, j, t) < j;
+            }
+            if (ok) pent[fill + rank] = (uint16_t)j;
+          }
+        } else {
+          // wide window: partners appended unordered to scratch (the score slots of this chunk's tail are free until
+          // B-score), then placed by rank
+          uint16_t *tmp = reinterpret_cast<uint16_t *>(psc + fill);
+          bool fits = true;
+          for (int tb = 0; tb < W_r; tb += 32) {
+            const int t = tb + lane;
+            int j = 0;
+            bool ok = false;
+            if (t < W_r) {
+              j = sidx[lo_r + t];
+              const float4 gj = *reinterpret_cast<const float4 *>(&sl.gatef[j].dx);
+              const int imgj = sl.gatef[j].img;
+              ok = (imgj != __float_as_int(a1.w)) && !(fabsf(gj.w - a0.w) > a1.z) &&
+                   !(fabsf(a0.x * gj.x + a0.y * gj.y + a0.z * gj.z) < p.cos_th3d_f);
+            }
+            const unsigned m = __ballot_sync(FULL, ok);
+            if (fill + n_r + __popc(m) > p.cap) { fits = false; break; }
+            if (ok) tmp[n_r + __popc(m & lt_mask)] = (uint16_t)j;
+            n_r += __popc(m);
+          }
+          if (!fits) break;
+          __syncwarp();
+          // (tmp occupies 2 bytes per partner inside psc[fill ..), pent[fill ..) is a different array)
+          for (int e = lane; e < n_r; e += 32) {
+            const uint16_t v = tmp[e];
+            int rank = 0;
+            for (int x = 0; x < n_r; ++x) rank += tmp[x] < v;
+            pent[fill + rank] = v;
+          }
+        }
+        if (lane == rr) { off = fill; n = n_r; }
+        fill += n_r;
+      }
+      const int ce = rr;
+      n1_total += (unsigned long long)fill;
+      __syncwarp();
+      // B-score: exact reference scores, lane = pair
+      for (int fb = 0; fb < fill; fb += 32) {
+        const int f = fb + lane;
+        int r = cb; // largest row of the chunk whose offset is <= f (rows without partners share the next offset)
+#pragma unroll
+        for (int step = 16; step >= 1; step >>= 1) {
+          const int cand = r + step;
+          const int v = __shfl_sync(FULL, off, cand & 31);
+          if (cand < ce && v <= f) r = cand;
+        }
+        if (f < fill) {
+          const int j = pent[f];
+          psc[f] = pair_score_fast<SPLIT>(p, sl, g0 + r, j, (uint32_t)sl.gatef[j].img);
+        }
+      }
+      n2_total += (unsigned long long)fill;
+      __syncwarp();
+      // B-sum: one image contributes its maximum once (:110-112), images in ascending order (the partners of a row
+      // are sorted by candidate index, i.e. by image)
+      if (lane >= cb && lane < ce) {
+        double sum = 0.0, mx = 0.0;
+        int cur = -1;
+        for (int e = 0; e < n; ++e) {
+          const int im = sl.gatef[pent[off + e]].img;
+          const double sc = psc[off + e];
+          if (im != cur) { sum += mx; cur = im; mx = sc; }
+          else mx = (mx > sc) ? mx : sc;
+        }
+        sum += mx;
+        sl.score[g0 + lane] = sum;
+      }
+      __syncwarp();
+    }
+  }
+}
+
+// Phase C: valid connections + best candidate (:115-153) of the node whose rows start at r0. slot0 is the record slot
+// of the node's first row (split path only).
+template <int NS, bool SPLIT>
+LM_D void phase_c(const TriParams &p, const Slab &sl, const int C, const uint32_t r0, NodeRecord *rec, int &s_nvalid,
+                  int64_t slot0 = 0) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int nvalid_local = 0;
+  for (int i = tid; i < C; i += kThreads) {
+    const double sc = sl.score[i];
+    bool valid = sc >= p.fullscore_th; // `if (score < fullscore_th) continue;`
+    if (valid && C > p.max_valid_conns) {
+      // rank in the (score, tri_id) descending order of std::greater<pair<double,int>> (:128-129)
+      int rank = 0;
+      for (int k = 0; k < C; ++k) {
+        const double sk = sl.score[k];
+        rank += (sk > sc) || (sk == sc && k > i);
+      }
+      valid = rank < p.max_valid_conns;
+    }
+    p.row_state[(int64_t)r0 * NS + sl.row[i]] = valid ? 2 : 1;
+    nvalid_local += valid;
+    if (p.row_cand) {
+      double *o = p.row_cand + ((int64_t)r0 * NS + sl.row[i]) * 10;
+      o[0] = sl.sx[i]; o[1] = sl.sy[i]; o[2] = sl.sz[i]; o[3] = sl.ex[i]; o[4] = sl.ey[i]; o[5] = sl.ez[i];
+      o[6] = cand_field<SPLIT>(p, sl, sl.zs, 6, i, slot0); o[7] = cand_field<SPLIT>(p, sl, sl.ze, 7, i, slot0);
+      o[8] = cand_field<SPLIT>(p, sl, sl.unc, 8, i, slot0); o[9] = sc;
+    }
+  }
+  if (nvalid_local) atomicAdd(&s_nvalid, nvalid_local);
+  // best: first strict maximum from max_score = -1 (:145-153) == max score, lowest index on ties.
+  if (warp == 0) {
+    double bs = -1.0;
+    int bi = -1;
+    for (int i = lane; i < C; i += 32) {
+      const double sc = sl.score[i];
+      if (sc > bs) { bs = sc; bi = i; }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+      const double os = __shfl_down_sync(0xffffffffu, bs, d);
+      const int oi = __shfl_down_sync(0xffffffffu, bi, d);
+      if (oi >= 0 && (os > bs || (os == bs && (bi < 0 || oi < bi)))) { bs = os; bi = oi; }
+    }
+    bi = __shfl_sync(0xffffffffu, bi, 0);
+    if (bi >= 0) {
+      if (lane < 3) rec->line[lane] = (lane == 0) ? sl.sx[bi] : (lane == 1 ? sl.sy[bi] : sl.sz[bi]);
+      else if (lane < 6) rec->line[lane] = (lane == 3) ? sl.ex[bi] : (lane == 4 ? sl.ey[bi] : sl.ez[bi]);
+      else if (lane == 6) rec->line[6] = cand_field<SPLIT>(p, sl, sl.zs, 6, bi, slot0);
+      else if (lane == 7) rec->line[7] = cand_field<SPLIT>(p, sl, sl.ze, 7, bi, slot0);
+      else if (lane == 8) rec->line[8] = cand_field<SPLIT>(p, sl, sl.unc, 8, bi, slot0);
+      else if (lane == 9) rec->score = sl.score[bi];
+      else if (lane == 10) { rec->ng_view = (int32_t)(sl.ng[bi] >> 16); rec->ng_line = (int32_t)(sl.ng[bi] & 0xffffu); }
+    } else {
+      if (lane < 9) rec->line[lane] = (lane == 8) ? -1.0 : 0.0;
+      if (lane == 9) rec->score = 0.0;
+      if (lane == 10) { rec->ng_view = 0; rec->ng_line = 0; }
+    }
+  }
 }
 
 // FAST: reduced-form scorer and plane-pair triangulation only (the default configuration); the generic
@@ -773,50 +1092,7 @@ __global__ void __launch_bounds__(kThreads, LM_TRI_MIN_BLOCKS) tri_node_kernel(c
 #pragma unroll
       for (int k = 0; k < NS; ++k) {
         if (!oks[k]) continue;
-        const Cand &c = cs[k];
-        const vec3<double> dr = c.e - c.s;
-        const double dn2 = dot(dr, dr);
-        const vec3<double> d = (dn2 > 0.0) ? dr * (1.0 / sqrt(dn2)) : dr;
-        sl.sx[idx] = c.s.x; sl.sy[idx] = c.s.y; sl.sz[idx] = c.s.z;
-        sl.ex[idx] = c.e.x; sl.ey[idx] = c.e.y; sl.ez[idx] = c.e.z;
-        sl.dx[idx] = d.x; sl.dy[idx] = d.y; sl.dz[idx] = d.z;
-        sl.zs[idx] = c.zs; sl.ze[idx] = c.ze; sl.unc[idx] = c.unc;
-        sl.q0[idx] = l2.x; sl.q1[idx] = l2.y; sl.q2[idx] = l2.z; sl.q3[idx] = l2.w;
-        if (FAST) {
-          const double zs1 = c.zs + consts<double>::eps(), ze1 = c.ze + consts<double>::eps();
-          const double qx = l2.z - l2.x, qy = l2.w - l2.y;
-          sl.izs2[idx] = 1.0 / (zs1 * zs1); sl.ize2[idx] = 1.0 / (ze1 * ze1); sl.inb[idx] = 1.0 / (qx * qx + qy * qy);
-        }
-        sl.ng[idx] = ng;
-        sl.row[idx] = (uint32_t)r * NS + k;
-        if (FAST) {
-          // fp32 gate record: the endpoints as distances along the two source rays. Limits: th * (z + EPS) widened by
-          // 0.5% plus 1e-5 of the larger distance (fp32 rounding of the two lambdas and of their difference is below
-          // 2e-7 of it, |X_i - X_j| and |lambda_i - lambda_j| agree to 1e-15); see DESIGN.md "gates"
-          const double rad = fmax(fabs(c.lam_s), fabs(c.lam_e));
-          const double ls = p.l3d.th_scaleinv * (c.zs + consts<double>::eps()) * 1.005 + 1e-5 * rad;
-          const double le = p.l3d.th_scaleinv * (c.ze + consts<double>::eps()) * 1.005 + 1e-5 * rad;
-          GateRecF g;
-          g.dx = (float)d.x; g.dy = (float)d.y; g.dz = (float)d.z; g.lam_e = (float)c.lam_e;
-          g.lam_s = (float)c.lam_s; g.lim_s = (float)(ls * 1.000001); g.lim_e = (float)(le * 1.000001);
-          g.img = (int)(ng >> 16);
-          sl.gatef[idx] = g;
-          reinterpret_cast<float *>(sl.psc)[idx] = g.lam_s; // unsorted keys of the depth sort (scratch: the score lists)
-        } else {
-          // fp32 gate copy, relative to the source camera centre (keeps |coord| ~ depth)
-          const vec3<double> rs = c.s - src.C1, re = c.e - src.C1;
-          // scale-invariance limit th * (z + EPS) widened by 0.5% plus 1e-5 of the coordinate magnitude
-          // (fp32 rounding of the two endpoints is < 1e-6 of it); see DESIGN.md "gates"
-          const double rad = sqrt(fmax(dot(rs, rs), dot(re, re)));
-          const double ls = p.l3d.th_scaleinv * (c.zs + consts<double>::eps()) * 1.005 + 1e-5 * rad;
-          const double le = p.l3d.th_scaleinv * (c.ze + consts<double>::eps()) * 1.005 + 1e-5 * rad;
-          GateRec g;
-          g.dx = (float)d.x; g.dy = (float)d.y; g.dz = (float)d.z; g.lims2 = (float)(ls * ls * 1.000001);
-          g.sx = (float)rs.x; g.sy = (float)rs.y; g.sz = (float)rs.z; g.lime2 = (float)(le * le * 1.000001);
-          g.ex = (float)re.x; g.ey = (float)re.y; g.ez = (float)re.z;
-          g.pad = 0.f;
-          sl.gate[idx] = g;
-        }
+        stage_cand<FAST, false>(p, sl, idx, cs[k], l2, ng, (uint32_t)r * NS + k, src.C1);
         ++idx;
       }
       count += tot;
@@ -840,161 +1116,7 @@ __global__ void __launch_bounds__(kThreads, LM_TRI_MIN_BLOCKS) tri_node_kernel(c
       //            reference's std::map (:105-112), so a row's total does not depend on how the work was split.
       // Pruned pairs would have scored exactly 0 (DESIGN.md "Exactness argument"); every surviving pair is scored by
       // pair_score_fast in fp64.
-      const unsigned FULL = 0xffffffffu;
-      {
-        float *ltmp = reinterpret_cast<float *>(sl.psc);
-        const int C4 = (C + 3) & ~3;
-        if (tid < C4 - C) ltmp[C + tid] = __int_as_float(0x7f800000); // +inf pads: never below a key, never tie-winners
-        __syncthreads();
-        for (int i = tid; i < C; i += kThreads) {
-          const float li = ltmp[i];
-          int r = 0;
-          for (int j4 = 0; j4 < C4; j4 += 4) {
-            const float4 v = *reinterpret_cast<const float4 *>(ltmp + j4);
-            r += (v.x < li) || (v.x == li && j4 < i);
-            r += (v.y < li) || (v.y == li && j4 + 1 < i);
-            r += (v.z < li) || (v.z == li && j4 + 2 < i);
-            r += (v.w < li) || (v.w == li && j4 + 3 < i);
-          }
-          sl.slam[r] = li;
-          sl.sidx[r] = (uint16_t)i;
-        }
-        __syncthreads(); // ltmp (= the score lists) is dead from here on
-      }
-      const float *slam = sl.slam;
-      const uint16_t *sidx = sl.sidx;
-      double *psc = sl.psc + (size_t)warp * p.cap;
-      uint16_t *pent = sl.pent + (size_t)warp * p.cap;
-      // rows are dealt to the warps in equal shares (C = 100: 25 rows per warp, not 32 + 32 + 32 + 4), so the warps
-      // reach the barrier before phase C together
-      const int n_pass = (C + 32 * kWarps - 1) / (32 * kWarps);
-      const int G = (C + kWarps * n_pass - 1) / (kWarps * n_pass); // rows per warp and pass, <= 32
-      for (int pass = 0; pass < n_pass; ++pass) {
-        const int g0 = (pass * kWarps + warp) * G;
-        if (g0 >= C) break;
-        const int Gact = min(G, C - g0);
-        // B-window, lane = row: two binary searches over the sorted start distances
-        int lo = 0, W = 0;
-        if (lane < Gact) {
-          const float4 a1 = *reinterpret_cast<const float4 *>(&sl.gatef[g0 + lane].lam_s);
-          int hi = C;
-          if (a1.y < 3e37f) { // (false for inf / NaN limits: the whole node is the window then)
-            const float wa = a1.x - a1.y, wb = a1.x + a1.y;
-            int l = 0, h = C;
-            while (l < h) { const int m = (l + h) >> 1; if (slam[m] < wa) l = m + 1; else h = m; }
-            lo = l;
-            h = C;
-            while (l < h) { const int m = (l + h) >> 1; if (!(slam[m] > wb)) l = m + 1; else h = m; }
-            hi = l;
-          }
-          W = hi - lo;
-        }
-        int rr = 0;
-        while (rr < Gact) {
-          // B-gate, one row at a time, lane = window position: the other fp32 gates (end-point interval, angle, other
-          // image). The partners of a row are written in ascending candidate order (= ascending neighbour image:
-          // candidates are generated image by image) at the running fill of the warp's pair list; lane r keeps the
-          // offset and the count of row r of the chunk. A chunk ends when the next row would not fit the list.
-          const int cb = rr;
-          int fill = 0, off = 0, n = 0;
-          for (; rr < Gact; ++rr) {
-            const int lo_r = __shfl_sync(FULL, lo, rr), W_r = __shfl_sync(FULL, W, rr);
-            const float4 a0 = *reinterpret_cast<const float4 *>(&sl.gatef[g0 + rr].dx);
-            const float4 a1 = *reinterpret_cast<const float4 *>(&sl.gatef[g0 + rr].lam_s);
-            int n_r = 0;
-            if (W_r <= 32) {
-              int j = 0x7fffffff;
-              bool ok = false;
-              if (lane < W_r) {
-                j = sidx[lo_r + lane];
-                const float4 gj = *reinterpret_cast<const float4 *>(&sl.gatef[j].dx);
-                const int imgj = sl.gatef[j].img;
-                ok = (imgj != __float_as_int(a1.w)) && !(fabsf(gj.w - a0.w) > a1.z) &&
-                     !(fabsf(a0.x * gj.x + a0.y * gj.y + a0.z * gj.z) < p.cos_th3d_f);
-              }
-              unsigned m = __ballot_sync(FULL, ok);
-              n_r = __popc(m);
-              if (n_r) {
-                if (fill + n_r > p.cap) break; // (a row has fewer than C <= cap partners: an empty list always takes it)
-                int rank = 0;
-                while (m) { // rank among the partners by candidate index: n_r independent shuffles
-                  const int t = __ffs((int)m) - 1;
-                  m &= m - 1;
-                  rank += __shfl_sync(FULL, j, t) < j;
-                }
-                if (ok) pent[fill + rank] = (uint16_t)j;
-              }
-            } else {
-              // wide window: partners appended unordered to scratch (the score slots of this chunk's tail are free until
-              // B-score), then placed by rank
-              uint16_t *tmp = reinterpret_cast<uint16_t *>(psc + fill);
-              bool fits = true;
-              for (int tb = 0; tb < W_r; tb += 32) {
-                const int t = tb + lane;
-                int j = 0;
-                bool ok = false;
-                if (t < W_r) {
-                  j = sidx[lo_r + t];
-                  const float4 gj = *reinterpret_cast<const float4 *>(&sl.gatef[j].dx);
-                  const int imgj = sl.gatef[j].img;
-                  ok = (imgj != __float_as_int(a1.w)) && !(fabsf(gj.w - a0.w) > a1.z) &&
-                       !(fabsf(a0.x * gj.x + a0.y * gj.y + a0.z * gj.z) < p.cos_th3d_f);
-                }
-                const unsigned m = __ballot_sync(FULL, ok);
-                if (fill + n_r + __popc(m) > p.cap) { fits = false; break; }
-                if (ok) tmp[n_r + __popc(m & lt_mask)] = (uint16_t)j;
-                n_r += __popc(m);
-              }
-              if (!fits) break;
-              __syncwarp();
-              // (tmp occupies 2 bytes per partner inside psc[fill ..), pent[fill ..) is a different array)
-              for (int e = lane; e < n_r; e += 32) {
-                const uint16_t v = tmp[e];
-                int rank = 0;
-                for (int x = 0; x < n_r; ++x) rank += tmp[x] < v;
-                pent[fill + rank] = v;
-              }
-            }
-            if (lane == rr) { off = fill; n = n_r; }
-            fill += n_r;
-          }
-          const int ce = rr;
-          n1_total += (unsigned long long)fill;
-          __syncwarp();
-          // B-score: exact reference scores, lane = pair
-          for (int fb = 0; fb < fill; fb += 32) {
-            const int f = fb + lane;
-            int r = cb; // largest row of the chunk whose offset is <= f (rows without partners share the next offset)
-#pragma unroll
-            for (int step = 16; step >= 1; step >>= 1) {
-              const int cand = r + step;
-              const int v = __shfl_sync(FULL, off, cand & 31);
-              if (cand < ce && v <= f) r = cand;
-            }
-            if (f < fill) {
-              const int j = pent[f];
-              psc[f] = pair_score_fast(p, sl, g0 + r, j, (uint32_t)sl.gatef[j].img);
-            }
-          }
-          n2_total += (unsigned long long)fill;
-          __syncwarp();
-          // B-sum: one image contributes its maximum once (:110-112), images in ascending order (the partners of a row
-          // are sorted by candidate index, i.e. by image)
-          if (lane >= cb && lane < ce) {
-            double sum = 0.0, mx = 0.0;
-            int cur = -1;
-            for (int e = 0; e < n; ++e) {
-              const int im = sl.gatef[pent[off + e]].img;
-              const double sc = psc[off + e];
-              if (im != cur) { sum += mx; cur = im; mx = sc; }
-              else mx = (mx > sc) ? mx : sc;
-            }
-            sum += mx;
-            sl.score[g0 + lane] = sum;
-          }
-          __syncwarp();
-        }
-      }
+      phase_b_fast<false>(p, sl, C, n1_total, n2_total);
       __syncthreads();
     } else {
     // Warps fetch rows i dynamically. B1 prunes (i, j) pairs with the fp32 3d gates and appends the
@@ -1141,57 +1263,7 @@ __global__ void __launch_bounds__(kThreads, LM_TRI_MIN_BLOCKS) tri_node_kernel(c
     __syncthreads();
     } // generic phase B
     // ---------------- phase C: valid connections + best candidate (:115-153) ----------------
-    int nvalid_local = 0;
-    for (int i = tid; i < C; i += kThreads) {
-      const double sc = sl.score[i];
-      bool valid = sc >= p.fullscore_th; // `if (score < fullscore_th) continue;`
-      if (valid && C > p.max_valid_conns) {
-        // rank in the (score, tri_id) descending order of std::greater<pair<double,int>> (:128-129)
-        int rank = 0;
-        for (int k = 0; k < C; ++k) {
-          const double sk = sl.score[k];
-          rank += (sk > sc) || (sk == sc && k > i);
-        }
-        valid = rank < p.max_valid_conns;
-      }
-      p.row_state[(int64_t)r0 * NS + sl.row[i]] = valid ? 2 : 1;
-      nvalid_local += valid;
-      if (p.row_cand) {
-        double *o = p.row_cand + ((int64_t)r0 * NS + sl.row[i]) * 10;
-        o[0] = sl.sx[i]; o[1] = sl.sy[i]; o[2] = sl.sz[i]; o[3] = sl.ex[i]; o[4] = sl.ey[i]; o[5] = sl.ez[i];
-        o[6] = sl.zs[i]; o[7] = sl.ze[i]; o[8] = sl.unc[i]; o[9] = sc;
-      }
-    }
-    if (nvalid_local) atomicAdd(&s_nvalid, nvalid_local);
-    // best: first strict maximum from max_score = -1 (:145-153) == max score, lowest index on ties.
-    if (warp == 0) {
-      double bs = -1.0;
-      int bi = -1;
-      for (int i = lane; i < C; i += 32) {
-        const double sc = sl.score[i];
-        if (sc > bs) { bs = sc; bi = i; }
-      }
-#pragma unroll
-      for (int d = 16; d > 0; d >>= 1) {
-        const double os = __shfl_down_sync(0xffffffffu, bs, d);
-        const int oi = __shfl_down_sync(0xffffffffu, bi, d);
-        if (oi >= 0 && (os > bs || (os == bs && (bi < 0 || oi < bi)))) { bs = os; bi = oi; }
-      }
-      bi = __shfl_sync(0xffffffffu, bi, 0);
-      if (bi >= 0) {
-        if (lane < 3) rec->line[lane] = (lane == 0) ? sl.sx[bi] : (lane == 1 ? sl.sy[bi] : sl.sz[bi]);
-        else if (lane < 6) rec->line[lane] = (lane == 3) ? sl.ex[bi] : (lane == 4 ? sl.ey[bi] : sl.ez[bi]);
-        else if (lane == 6) rec->line[6] = sl.zs[bi];
-        else if (lane == 7) rec->line[7] = sl.ze[bi];
-        else if (lane == 8) rec->line[8] = sl.unc[bi];
-        else if (lane == 9) rec->score = sl.score[bi];
-        else if (lane == 10) { rec->ng_view = (int32_t)(sl.ng[bi] >> 16); rec->ng_line = (int32_t)(sl.ng[bi] & 0xffffu); }
-      } else {
-        if (lane < 9) rec->line[lane] = (lane == 8) ? -1.0 : 0.0;
-        if (lane == 9) rec->score = 0.0;
-        if (lane == 10) { rec->ng_view = 0; rec->ng_line = 0; }
-      }
-    }
+    phase_c<NS, false>(p, sl, C, r0, rec, s_nvalid);
     __syncthreads();
     if (tid == 0) {
       rec->n_cand = C;
@@ -1225,6 +1297,179 @@ cudaError_t launch_tri_node_kernel(const TriParams &p, int grid, int block, size
   const bool fast = p.fast_forms && !p.use_endpoints_triangulation;
   if (p.use_vp) return fast ? launch_tri_vf<true, true>(p, grid, smem, s) : launch_tri_vf<true, false>(p, grid, smem, s);
   return fast ? launch_tri_vf<false, true>(p, grid, smem, s) : launch_tri_vf<false, false>(p, grid, smem, s);
+}
+
+// ---- split fast path ------------------------------------------------------------------------------------------------
+// The fused kernel holds phase A's fp64 registers and the scorer's staging area in one CTA, which caps it at 4 CTAs/SM.
+// Split, each part runs at its own occupancy: generation is flat (one thread per match row, no shared memory, no
+// barriers) and writes each candidate as a record to global memory; scoring is one CTA per node sized from the real
+// candidate count. The same fp64 values cross the boundary and the same expressions run on them, so the results are
+// those of the fused kernel.
+#ifndef LM_GEN_THREADS
+#define LM_GEN_THREADS 128
+#endif
+#ifndef LM_SCORE_MIN_BLOCKS
+#define LM_SCORE_MIN_BLOCKS 6
+#endif
+
+// One thread per match row of the group: phase A of tri_node_kernel without the compaction. Writes row_state = 0 / 1
+// for every proposal slot and the record of every candidate.
+template <bool VP>
+__global__ void __launch_bounds__(LM_GEN_THREADS, VP ? 2 : 3) tri_gen_kernel(const __grid_constant__ TriParams p) {
+  constexpr int NS = VP ? 3 : 1;
+  const int64_t r = p.row_begin + blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (r >= p.row_end) return;
+  const uint32_t node = __ldg(&p.row_node[r]);
+  const uint32_t v1i = p.node_view[node];
+  const ViewD &v1 = p.views[v1i];
+  Src src;
+  src.l1 = ld_seg(&p.segs[node]);
+  {
+    double dx = src.l1.x - src.l1.z, dy = src.l1.y - src.l1.w;
+    src.ok = !(sqrt(dx * dx + dy * dy) <= p.min_length_2d); // :166
+    src.w1s = mat3_mul_h(v1.M, src.l1.x, src.l1.y);
+    src.w1e = mat3_mul_h(v1.M, src.l1.z, src.l1.w);
+    src.ray1s = normalized(src.w1s);
+    src.ray1e = normalized(src.w1e);
+    src.C1 = mk3(v1.C[0], v1.C[1], v1.C[2]);
+    src.n1 = normalized(cross(src.w1s, src.w1e));
+  }
+  Cand cs[NS];
+  bool oks[NS];
+#pragma unroll
+  for (int k = 0; k < NS; ++k) oks[k] = false;
+  if (src.ok) {
+    const uint32_t ng = __ldg(&p.row_ng[r]);
+    const uint32_t ngv = ng >> 16, ngl = ng & 0xffffu;
+    const ViewD &v2 = p.views[ngv];
+    double4 l2;
+    if (VP) {
+      // Step 2 (:258-288): proposals from the VP of the source line and of the matched line; both use view 1
+      const double4 l2v = ld_seg(&p.segs[p.line_off[ngv] + ngl]);
+      const double ddx = l2v.x - l2v.z, ddy = l2v.y - l2v.w;
+      if (!(sqrt(ddx * ddx + ddy * ddy) <= p.min_length_2d) && !p.disable_vp) {
+        const vec3<double> c2s = mat3_mul_h(v2.M, l2v.x, l2v.y), c2e = mat3_mul_h(v2.M, l2v.z, l2v.w);
+        const int lab1 = p.vp_label[node];
+        if (lab1 >= 0) {
+          const double *vp = p.vps + 3 * (p.vp_off[v1i] + lab1);
+          oks[0] = gen_vp_candidate(p, v1, v2, src, c2s, c2e, normalized(mat3_mul(v1.M, mk3(vp[0], vp[1], vp[2]))), cs[0]);
+        }
+        const int lab2 = p.vp_label[p.line_off[ngv] + ngl];
+        if (lab2 >= 0) {
+          const double *vp = p.vps + 3 * (p.vp_off[ngv] + lab2);
+          oks[1] = gen_vp_candidate(p, v1, v2, src, c2s, c2e, normalized(mat3_mul(v1.M, mk3(vp[0], vp[1], vp[2]))), cs[1]);
+        }
+      }
+    }
+    oks[NS - 1] = gen_candidate<false>(p, v1, v2, src, ngv, ngl, cs[NS - 1], l2);
+  }
+  const int64_t q0 = (r - p.row_begin) * NS;
+#pragma unroll
+  for (int k = 0; k < NS; ++k) {
+    p.row_state[r * NS + k] = oks[k] ? 1 : 0;
+    if (!oks[k]) continue;
+    const Cand &c = cs[k];
+    double *o = p.cand + q0 + k;
+    const int64_t st = p.cand_stride;
+    o[0] = c.s.x; o[st] = c.s.y; o[2 * st] = c.s.z; o[3 * st] = c.e.x; o[4 * st] = c.e.y; o[5 * st] = c.e.z;
+    o[6 * st] = c.zs; o[7 * st] = c.ze; o[8 * st] = c.unc; o[9 * st] = c.lam_s; o[10 * st] = c.lam_e;
+  }
+}
+
+// One CTA per node: the node's candidate slots (row_state == 1) in slot order -- the order of the fused kernel's stable
+// compaction, so candidate indices are the same -- staged from their records, then phases B and C of the fused kernel.
+template <bool VP>
+__global__ void __launch_bounds__(kThreads, LM_SCORE_MIN_BLOCKS) tri_score_kernel(const __grid_constant__ TriParams p) {
+  constexpr int NS = VP ? 3 : 1;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ int s_wtot[kWarps];
+  __shared__ int s_nvalid;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const unsigned lt_mask = (1u << lane) - 1u;
+  Slab sl;
+  sl.carve_split(reinterpret_cast<char *>(smem_raw), p.cap);
+  unsigned long long n1_total = 0, n2_total = 0;
+  for (int64_t node = p.node_begin + blockIdx.x; node < p.node_end; node += gridDim.x) {
+    const uint32_t r0 = p.node_row_off[node], r1 = p.node_row_off[node + 1];
+    const int nslots = (int)(r1 - r0) * NS;
+    NodeRecord *rec = &p.nodes[node];
+    // compaction of the candidate slots
+    int count = 0;
+    for (int base = 0; base < nslots; base += kThreads) {
+      const int q = base + tid;
+      const bool cand = q < nslots && p.row_state[(int64_t)r0 * NS + q] == 1;
+      const unsigned m = __ballot_sync(0xffffffffu, cand);
+      if (lane == 0) s_wtot[warp] = __popc(m);
+      __syncthreads();
+      int woff = 0, tot = 0;
+#pragma unroll
+      for (int w = 0; w < kWarps; ++w) {
+        if (w < warp) woff += s_wtot[w];
+        tot += s_wtot[w];
+      }
+      const int idx = count + woff + __popc(m & lt_mask);
+      if (cand && idx < p.cap) sl.row[idx] = (uint32_t)q;
+      count += tot;
+      __syncthreads();
+    }
+    const int C = count;
+    if (tid == 0 && C) atomicMax(p.max_cand, (unsigned int)C);
+    if (C > p.cap) { // staging area sized from a stale hint: the host repeats the run with the exact size
+      if (tid < 9) rec->line[tid] = (tid == 8) ? -1.0 : 0.0;
+      if (tid == 9) { rec->score = 0.0; rec->ng_view = 0; rec->ng_line = 0; rec->n_cand = 0; rec->n_valid = 0; }
+      if (tid == 10) *p.overflow = 1;
+      continue;
+    }
+    // ---- staging from the records (phase A's derivation)
+    const int64_t slot0 = (int64_t)(r0 - p.row_begin) * NS;
+    for (int i = tid; i < C; i += kThreads) {
+      const uint32_t q = sl.row[i];
+      const double *o = p.cand + slot0 + q;
+      const int64_t st = p.cand_stride;
+      Cand c;
+      c.s = mk3(o[0], o[st], o[2 * st]);
+      c.e = mk3(o[3 * st], o[4 * st], o[5 * st]);
+      c.zs = o[6 * st]; c.ze = o[7 * st]; c.unc = o[8 * st]; c.lam_s = o[9 * st]; c.lam_e = o[10 * st];
+      const uint32_t ng = __ldg(&p.row_ng[r0 + q / NS]);
+      const uint32_t segi = (uint32_t)(p.line_off[ng >> 16] + (ng & 0xffffu));
+      stage_cand<true, true>(p, sl, i, c, ld_seg(&p.segs[segi]), ng, q, mk3(0.0, 0.0, 0.0), segi); // (C1: generic layout only)
+    }
+    if (tid == 0) s_nvalid = 0;
+    __syncthreads();
+    phase_b_fast<true>(p, sl, C, n1_total, n2_total);
+    __syncthreads();
+    phase_c<NS, true>(p, sl, C, r0, rec, s_nvalid, slot0);
+    __syncthreads();
+    if (tid == 0) {
+      rec->n_cand = C;
+      rec->n_valid = s_nvalid;
+      if (C) atomicAdd(&p.counters[0], (unsigned long long)C);
+      if (s_nvalid) atomicAdd(&p.counters[1], (unsigned long long)s_nvalid);
+    }
+    __syncthreads();
+  }
+  if (lane == 0 && n1_total) {
+    atomicAdd(&p.counters[2], n1_total); // pairs past the fp32 3d gates
+    atomicAdd(&p.counters[3], n2_total); // pairs scored exactly in fp64
+  }
+}
+
+template <bool VP> static cudaError_t launch_split_v(const TriParams &p, int grid, size_t smem, cudaStream_t s) {
+  const int64_t rows = p.row_end - p.row_begin;
+  if (rows > 0) {
+    tri_gen_kernel<VP><<<(unsigned)((rows + LM_GEN_THREADS - 1) / LM_GEN_THREADS), LM_GEN_THREADS, 0, s>>>(p);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+  }
+  if (smem > 48 * 1024) {
+    const cudaError_t e = cudaFuncSetAttribute(tri_score_kernel<VP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  tri_score_kernel<VP><<<grid, kThreads, smem, s>>>(p);
+  return cudaGetLastError();
+}
+cudaError_t launch_tri_split(const TriParams &p, int grid, size_t smem, cudaStream_t s) {
+  return p.use_vp ? launch_split_v<true>(p, grid, smem, s) : launch_split_v<false>(p, grid, smem, s);
 }
 
 // The per-run block tables (match tables ordered by (source view, neighbour), row offsets) are derived on the

@@ -47,6 +47,12 @@ struct TriParams {
   int64_t node_begin, node_end;
   int cap;                     // candidate capacity of the staging area
   int use_slab;
+  // split path (tri_gen_kernel + tri_score_kernel) of one pipeline group
+  const uint32_t *row_node;    // [rows] node of every row (the node-sorted keys)
+  double *cand;                // candidate records of the group's slots, field-major (see tri_kernels.cu)
+  int64_t cand_stride;         // slots per field
+  int64_t row_begin, row_end;  // rows of the group
+  unsigned int *max_cand;      // largest candidate count of a node in the run
   // config (triangulation/base_line_triangulator.h:22-43, global_line_triangulator.h:11-25)
   double min_length_2d, line_tri_angle_threshold, IoU_threshold, sensitivity_threshold, var2d, fullscore_th;
   int max_valid_conns, use_endpoints_triangulation, disable_algebraic, use_vp, disable_vp;
@@ -84,6 +90,10 @@ void launch_group_edges(const uint8_t *row_state, const uint32_t *row_ng, const 
 void launch_scene_prepare(const double *segs_raw, int64_t n_nodes, double add, const int64_t *line_off, int n_views,
                           double *segs, uint16_t *node_view, cudaStream_t s);
 cudaError_t launch_tri_node_kernel(const TriParams &p, int grid, int block, size_t smem, cudaStream_t s);
+// Split form of the fast path: candidates of all rows of the group, then per-node scoring (p.cap sized from candidates).
+static constexpr int kCandFields = 11; // fp64 fields of a candidate record
+size_t tri_score_smem_bytes(int cap);
+cudaError_t launch_tri_split(const TriParams &p, int grid, size_t smem, cudaStream_t s);
 void launch_expand_rows(const int32_t *d_pairs, const int64_t *d_blk_row_off, const int32_t *d_blk_src_view,
                         const int32_t *d_blk_ng_view, const int64_t *d_blk_pair_off, int n_blocks,
                         const int64_t *d_line_off, int64_t r_begin, int64_t r_end, uint32_t *d_key, uint32_t *d_val,
