@@ -183,7 +183,8 @@ struct lm_ctx {
   unsigned int *h_pin = nullptr;
   // run buffers
   DevBuf d_blk_row_off, d_blk_src, d_blk_ng, d_blk_pair_off;
-  DevBuf d_key, d_key2, d_val, d_val2, d_sort_tmp;
+  DevBuf d_key, d_key2, d_val, d_val2, d_sort_tmp; // d_key / d_val: unsorted rows of the radix-sort path only
+  DevBuf d_rs_vrow, d_rs_vtile, d_rs_vtab, d_rs_tab;  // counting-sort row preparation: per-view tables, tile table
   DevBuf d_node_row_off, d_scalars; // scalars: [0] max_rows(uint) [1] err(int) ; counters at +16
   DevBuf d_nodes, d_row_state, d_row_cand, d_slab, d_cand;
   DevBuf d_edges, d_edges2, d_edge_keys, d_edge_keys2, d_edge_w, d_edge_cnt;
@@ -330,6 +331,7 @@ void lm_ctx_destroy(lm_ctx *c) {
   cudaStreamSynchronize(c->stream);
   DevBuf *bufs[] = {&c->d_scan_tmp, &c->d_local_off, &c->d_segs_raw, &c->d_img_ids, &c->d_host_edges, &c->d_views, &c->d_segs, &c->d_node_view, &c->d_line_off, &c->d_pairs, &c->d_blk_row_off,
                     &c->d_blk_src, &c->d_blk_ng, &c->d_blk_pair_off, &c->d_key, &c->d_key2, &c->d_val, &c->d_val2,
+                    &c->d_rs_vrow, &c->d_rs_vtile, &c->d_rs_vtab, &c->d_rs_tab,
                     &c->d_sort_tmp, &c->d_node_row_off, &c->d_scalars, &c->d_nodes, &c->d_row_state, &c->d_row_cand,
                     &c->d_slab, &c->d_cand, &c->d_edges, &c->d_edges2, &c->d_edge_keys, &c->d_edge_keys2, &c->d_edge_w,
                     &c->d_edge_cnt, &c->d_nvalid, &c->d_edge_off, &c->d_edge_ng, &c->d_ba_in, &c->d_ba_blocks, &c->d_ba_out, &c->d_raw_blocks, &c->d_bkey, &c->d_bkey2, &c->d_bval, &c->d_bval2, &c->d_blk_rows, &c->d_vp_label, &c->d_vp_voff, &c->d_vp_vps, &c->d_vp_pts, &c->d_vp_off, &c->d_vp_labels, &c->d_vp_nc, &c->d_vp_ps, &c->d_vp_mat, &c->d_mg_in, &c->d_mg_out, &c->d_mg_edges, &c->d_gather, &c->d_vp_idx, &c->d_sfm_in, &c->d_sfm_keys, &c->d_sfm_keys2, &c->d_sfm_a, &c->d_sfm_b, &c->d_sfm_c, &c->d_sfm_d, &c->d_g_flag, &c->d_g_pos, &c->d_g_kc, &c->d_g_wc, &c->d_g_occ, &c->d_g_occ2, &c->d_g_hk, &c->d_g_hk2, &c->d_g_gidx, &c->d_g_gnode, &c->d_g_k1, &c->d_g_k1b, &c->d_g_k2, &c->d_g_k2b};
@@ -799,9 +801,7 @@ int lm_tri_run(lm_ctx *c) {
   CU(c->d_blk_src.ensure(4 * std::max(nb + 1, 2)));
   CU(c->d_blk_ng.ensure(4 * std::max(nb + 1, 2)));
   CU(c->d_blk_pair_off.ensure(8 * std::max(nb, 1)));
-  CU(c->d_key.ensure(4 * std::max<int64_t>(n_rows, 1)));
   CU(c->d_key2.ensure(4 * std::max<int64_t>(n_rows, 1)));
-  CU(c->d_val.ensure(4 * std::max<int64_t>(n_rows, 1)));
   CU(c->d_val2.ensure(4 * std::max<int64_t>(n_rows, 1)));
   CU(c->d_node_row_off.ensure(4 * (c->n_nodes + 2)));
   CU(c->d_scalars.ensure(1024));
@@ -992,6 +992,55 @@ int lm_tri_run(lm_ctx *c) {
     gb[g + 1] = bg1;
     max_group_rows = std::max(max_group_rows, row_off[bg1] - row_off[gb[g]]);
   }
+  // Node-major rows: a per-view stable counting sort (row_count / row_scan / row_scatter) by default; views with more
+  // than kRowSortMaxLines lines, exhaustive matching and LIMAP_B200_ROW_SORT=cub (read per run) take the radix-sort
+  // path (expand_rows -> stable radix sort by node id -> node_offsets). Both give the same rows and node offsets.
+  const char *row_sort_env = getenv("LIMAP_B200_ROW_SORT");
+  const bool row_sort_cub = exhaustive || (row_sort_env && !strcmp(row_sort_env, "cub"));
+  const int nvs = ve - vb;
+  // host copy of what row_views_kernel derives on the device: first row and first tile of every view of the shard
+  std::vector<int64_t> vrow(nvs + 1, 0);
+  std::vector<int32_t> vtile(nvs + 1, 0);
+  bool any_radix_rows = row_sort_cub && n_rows > 0;
+  if (!row_sort_cub) {
+    for (int i = 0; i < nb; ++i) vrow[blk[i].src_view - vb + 1] += blk[i].n_rows;
+    int64_t tab_words = 0;
+    for (int i = 0; i < nvs; ++i) {
+      const int64_t L = c->line_off[vb + i + 1] - c->line_off[vb + i], rows = vrow[i + 1];
+      const int64_t nt = L <= lm::kRowSortMaxLines ? (rows + lm::kRowSortTile - 1) / lm::kRowSortTile : 0;
+      if (L > lm::kRowSortMaxLines && rows > 0) any_radix_rows = true;
+      vtile[i + 1] = vtile[i] + (int32_t)nt;
+      tab_words += nt * std::max<int64_t>(L, 1);
+      vrow[i + 1] += vrow[i];
+    }
+    CU(c->d_rs_vrow.ensure(8 * (nvs + 1)));
+    CU(c->d_rs_vtile.ensure(4 * (nvs + 1)));
+    CU(c->d_rs_vtab.ensure(8 * (nvs + 1)));
+    CU(c->d_rs_tab.ensure(4 * std::max<int64_t>(tab_words, 1)));
+    lm::launch_row_views(c->d_blk_row_off.as<int64_t>(), c->d_blk_src.as<int32_t>(), nb, c->d_line_off.as<int64_t>(), vb,
+                         nvs, c->d_rs_vrow.as<int64_t>(), c->d_rs_vtile.as<int32_t>(), c->d_rs_vtab.as<int64_t>(), sp);
+    ++launches;
+  }
+  if (any_radix_rows) {
+    CU(c->d_key.ensure(4 * std::max<int64_t>(n_rows, 1)));
+    CU(c->d_val.ensure(4 * std::max<int64_t>(n_rows, 1)));
+  }
+  // stable LSD radix sort by node id of rows [r0, r1) into d_key2 / d_val2 keeps (neighbour, row) order inside every node
+  auto radix_sort_rows = [&](int64_t r0, int64_t r1) -> cudaError_t {
+    cub::DoubleBuffer<uint32_t> dk(c->d_key.as<uint32_t>() + r0, c->d_key2.as<uint32_t>() + r0);
+    cub::DoubleBuffer<uint32_t> dv(c->d_val.as<uint32_t>() + r0, c->d_val2.as<uint32_t>() + r0);
+    size_t tmp = 0;
+    cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, tmp, dk, dv, (int)(r1 - r0), 0, nbits, sp);
+    if (e == cudaSuccess) e = c->d_sort_tmp.ensure(tmp);
+    if (e == cudaSuccess) e = cub::DeviceRadixSort::SortPairs(c->d_sort_tmp.p, tmp, dk, dv, (int)(r1 - r0), 0, nbits, sp);
+    launches += (nbits + 7) / 8 + 1;
+    if (e == cudaSuccess && dk.Current() != c->d_key2.as<uint32_t>() + r0) {
+      e = cudaMemcpyAsync(c->d_key2.as<uint32_t>() + r0, dk.Current(), 4 * (r1 - r0), cudaMemcpyDeviceToDevice, sp);
+      if (e == cudaSuccess)
+        e = cudaMemcpyAsync(c->d_val2.as<uint32_t>() + r0, dv.Current(), 4 * (r1 - r0), cudaMemcpyDeviceToDevice, sp);
+    }
+    return e;
+  };
   if (split) {
     p.row_node = c->sorted_key;
     p.cand_stride = std::max<int64_t>(max_group_rows * ns, 1);
@@ -1016,33 +1065,53 @@ int lm_tri_run(lm_ctx *c) {
         if (ch.row_end >= need) { CU(cudaStreamWaitEvent(sp, ch.ev, 0)); break; }
     }
     unsigned int *d_max_rows = c->d_scalars.as<unsigned int>() + 16 + g;
-    if (re > rb) {
-      if (exhaustive)
-        lm::launch_expand_exhaustive(c->d_blk_row_off.as<int64_t>(), c->d_blk_src.as<int32_t>(), c->d_blk_ng.as<int32_t>(),
-                                     nb, c->d_line_off.as<int64_t>(), n_rows, c->d_key.as<uint32_t>(),
-                                     c->d_val.as<uint32_t>(), sp);
-      else
-        lm::launch_expand_rows(c->d_pairs.as<int32_t>(), c->d_blk_row_off.as<int64_t>(), c->d_blk_src.as<int32_t>(),
-                               c->d_blk_ng.as<int32_t>(), c->d_blk_pair_off.as<int64_t>(), nb,
-                               c->d_line_off.as<int64_t>(), rb, re, c->d_key.as<uint32_t>(), c->d_val.as<uint32_t>(),
-                               d_err, sp);
+    if (row_sort_cub) {
+      if (re > rb) {
+        if (exhaustive)
+          lm::launch_expand_exhaustive(c->d_blk_row_off.as<int64_t>(), c->d_blk_src.as<int32_t>(),
+                                       c->d_blk_ng.as<int32_t>(), nb, c->d_line_off.as<int64_t>(), n_rows,
+                                       c->d_key.as<uint32_t>(), c->d_val.as<uint32_t>(), sp);
+        else
+          lm::launch_expand_rows(c->d_pairs.as<int32_t>(), c->d_blk_row_off.as<int64_t>(), c->d_blk_src.as<int32_t>(),
+                                 c->d_blk_ng.as<int32_t>(), c->d_blk_pair_off.as<int64_t>(), nb,
+                                 c->d_line_off.as<int64_t>(), rb, re, c->d_key.as<uint32_t>(), c->d_val.as<uint32_t>(),
+                                 d_err, sp);
+        ++launches;
+        CU(radix_sort_rows(rb, re));
+      }
+      lm::launch_node_offsets(c->sorted_key + rb, re - rb, rb, node_lo, node_hi, c->d_node_row_off.as<uint32_t>(),
+                              d_max_rows, sp);
       ++launches;
-      // stable LSD radix sort by node id keeps (neighbour, row) order inside every node
-      cub::DoubleBuffer<uint32_t> dk(c->d_key.as<uint32_t>() + rb, c->d_key2.as<uint32_t>() + rb);
-      cub::DoubleBuffer<uint32_t> dv(c->d_val.as<uint32_t>() + rb, c->d_val2.as<uint32_t>() + rb);
-      size_t tmp = 0;
-      CU(cub::DeviceRadixSort::SortPairs(nullptr, tmp, dk, dv, (int)(re - rb), 0, nbits, sp));
-      CU(c->d_sort_tmp.ensure(tmp));
-      CU(cub::DeviceRadixSort::SortPairs(c->d_sort_tmp.p, tmp, dk, dv, (int)(re - rb), 0, nbits, sp));
-      launches += (nbits + 7) / 8 + 1;
-      if (dk.Current() != c->d_key2.as<uint32_t>() + rb) {
-        CU(cudaMemcpyAsync(c->d_key2.as<uint32_t>() + rb, dk.Current(), 4 * (re - rb), cudaMemcpyDeviceToDevice, sp));
-        CU(cudaMemcpyAsync(c->d_val2.as<uint32_t>() + rb, dv.Current(), 4 * (re - rb), cudaMemcpyDeviceToDevice, sp));
+    } else {
+      const int i_lo = gv0 - vb, i_hi = gv1 - vb, n_tiles = vtile[i_hi] - vtile[i_lo];
+      int max_lines = 0;
+      for (int i = i_lo; i < i_hi; ++i) {
+        const int64_t L = c->line_off[vb + i + 1] - c->line_off[vb + i];
+        if (L <= lm::kRowSortMaxLines) max_lines = std::max(max_lines, (int)L);
+      }
+      CU(lm::launch_row_sort(c->d_pairs.as<int32_t>(), c->d_blk_row_off.as<int64_t>(), c->d_blk_ng.as<int32_t>(),
+                             c->d_blk_pair_off.as<int64_t>(), nb, c->d_line_off.as<int64_t>(), vb,
+                             c->d_rs_vrow.as<int64_t>(), c->d_rs_vtile.as<int32_t>(), c->d_rs_vtab.as<int64_t>(), i_lo,
+                             i_hi, vtile[i_lo], n_tiles, max_lines, c->d_rs_tab.as<uint32_t>(),
+                             c->d_node_row_off.as<uint32_t>(), d_max_rows, c->d_key2.as<uint32_t>(),
+                             c->d_val2.as<uint32_t>(), d_err, sp));
+      launches += (i_hi > i_lo) + (n_tiles > 0 ? 2 : 0);
+      for (int i = i_lo; i < i_hi; ++i) { // views with too many lines for the shared-memory histograms
+        const int64_t n0 = c->line_off[vb + i], n1 = c->line_off[vb + i + 1];
+        if (n1 - n0 <= lm::kRowSortMaxLines) continue;
+        const int64_t r0 = vrow[i], r1 = vrow[i + 1];
+        if (r1 > r0) {
+          lm::launch_expand_rows(c->d_pairs.as<int32_t>(), c->d_blk_row_off.as<int64_t>(), c->d_blk_src.as<int32_t>(),
+                                 c->d_blk_ng.as<int32_t>(), c->d_blk_pair_off.as<int64_t>(), nb,
+                                 c->d_line_off.as<int64_t>(), r0, r1, c->d_key.as<uint32_t>(), c->d_val.as<uint32_t>(),
+                                 d_err, sp);
+          ++launches;
+          CU(radix_sort_rows(r0, r1));
+        }
+        lm::launch_node_offsets(c->sorted_key + r0, r1 - r0, r0, n0, n1, c->d_node_row_off.as<uint32_t>(), d_max_rows, sp);
+        ++launches;
       }
     }
-    lm::launch_node_offsets(c->sorted_key + rb, re - rb, rb, node_lo, node_hi, c->d_node_row_off.as<uint32_t>(),
-                            d_max_rows, sp);
-    ++launches;
     CU(cudaEventRecord(c->evp[g], sp));
     CU(cudaStreamWaitEvent(s, c->evp[g], 0));
     p.node_begin = node_lo;

@@ -5,7 +5,9 @@
 //       GlobalLineTriangulator::scoreOneNode       (triangulation/global_line_triangulator.cc:71-161)
 //     so that the candidate set of a node lives only in shared memory: match rows are read once from
 //     HBM, candidates are never written back unless debug_mode asks for them.
-//   expand_rows / node_offsets : turn the per-(image, neighbour) match tables into node-major rows.
+//   row_count / row_scan / row_scatter : turn the per-(image, neighbour) match tables into node-major rows (per-view
+//       stable counting sort); expand_rows / node_offsets + a radix sort do it for views with many lines and for
+//       exhaustive matching.
 //   collect_edges / edge_weights : run_clustering's edge list and 3d scores
 //       (global_line_triangulator.cc:234-291).
 //
@@ -13,7 +15,9 @@
 // the contract is bit-exact candidate indices); fp32 appears only in pruning gates with explicit margins
 // (see DESIGN.md "Precision").
 #include "tri_kernels.cuh"
+#include <algorithm>
 #include <cstdio>
+#include <cub/block/block_scan.cuh>
 
 namespace lm {
 
@@ -1612,6 +1616,274 @@ void launch_node_offsets(const uint32_t *d_sorted_key, int64_t n_rows, int64_t r
   const int grid = (int)((node_hi - node_lo + 1 + 255) / 256);
   node_offsets_kernel<<<grid, 256, 0, s>>>(d_sorted_key, n_rows, row_base, node_lo, node_hi, d_node_row_off,
                                            d_max_rows);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Node-major rows by a per-view stable counting sort. The rows of a view are contiguous in flat order and its nodes are
+// contiguous (line_off), so "stable sort by node id" is a stable partition of each view's rows by local line id. A view's
+// rows are cut into tiles of kRowSortTile rows (never straddling a view); each tile histograms its lines (row_count),
+// an exclusive prefix over the tiles of every (view, line) gives each tile's slot per line and the node row offsets
+// (row_scan), and each tile writes its rows to their slots in row order (row_scatter). The result is the one a stable
+// sort gives: d_key2/d_val2 and node_row_off byte for byte as the radix-sort path (expand_rows -> sort -> node_offsets).
+static constexpr int kRowSortThreads = 256;
+static constexpr int kRowSortWarps = kRowSortThreads / 32;
+static constexpr int kRowSortSlice = kRowSortTile / kRowSortWarps; // contiguous rows per warp in row_scatter
+
+// Per view i of the shard (view vb + i): first row vrow[i] (vrow[nvs] = rows of the shard), first tile vtile[i] and
+// first tile-table word vtab[i] (a view's table is [tile][max(L, 1)]). Views above kRowSortMaxLines get no tiles.
+// One CTA for the whole shard; the host derives the same numbers from its copy of the block table.
+__global__ void row_views_kernel(const int64_t *__restrict__ blk_row_off, const int32_t *__restrict__ blk_src, int nb,
+                                 const int64_t *__restrict__ line_off, int vb, int nvs, int64_t *__restrict__ vrow,
+                                 int32_t *__restrict__ vtile, int64_t *__restrict__ vtab) {
+  typedef cub::BlockScan<int64_t, kRowSortThreads> Scan;
+  __shared__ typename Scan::TempStorage ts;
+  __shared__ int64_t carry[2];
+  if (threadIdx.x == 0) carry[0] = carry[1] = 0;
+  __syncthreads();
+  auto first_row = [&](int v) { // row offset of the first block with src_view >= v
+    int lo = 0, hi = nb;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (blk_src[mid] < v) lo = mid + 1; else hi = mid;
+    }
+    return blk_row_off[lo];
+  };
+  for (int i0 = 0; i0 <= nvs; i0 += kRowSortThreads) {
+    const int i = i0 + threadIdx.x;
+    int64_t nt = 0, nw = 0;
+    if (i <= nvs) {
+      const int64_t r0 = first_row(vb + i);
+      vrow[i] = r0;
+      if (i < nvs) {
+        const int64_t L = line_off[vb + i + 1] - line_off[vb + i];
+        if (L <= kRowSortMaxLines) {
+          nt = (first_row(vb + i + 1) - r0 + kRowSortTile - 1) / kRowSortTile;
+          nw = nt * (L > 0 ? L : 1);
+        }
+      }
+    }
+    int64_t et, ew, at, aw;
+    Scan(ts).ExclusiveSum(nt, et, at);
+    __syncthreads();
+    Scan(ts).ExclusiveSum(nw, ew, aw);
+    if (i <= nvs) {
+      vtile[i] = (int32_t)(carry[0] + et);
+      vtab[i] = carry[1] + ew;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) { carry[0] += at; carry[1] += aw; }
+    __syncthreads();
+  }
+}
+
+struct RowTile { // the tile a CTA of row_count / row_scatter works on
+  int64_t node0, r0, r1, tab; // first node of the view, rows [r0, r1), its table row
+  int L, Lb, b0, i;           // lines of the view, table stride max(L, 1), block of row r0, view index
+};
+__device__ __forceinline__ void row_tile_of(int tile, const int64_t *__restrict__ blk_row_off, int nb,
+                                            const int64_t *__restrict__ line_off, int vb, const int64_t *__restrict__ vrow,
+                                            const int32_t *__restrict__ vtile, const int64_t *__restrict__ vtab, int i_lo,
+                                            int i_hi, RowTile &rt) {
+  __shared__ RowTile s_rt;
+  if (threadIdx.x == 0) {
+    int lo = i_lo, hi = i_hi; // largest view i with vtile[i] <= tile (views without tiles are skipped)
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if (vtile[mid] <= tile) lo = mid; else hi = mid;
+    }
+    RowTile t;
+    t.i = lo;
+    t.node0 = line_off[vb + lo];
+    t.L = (int)(line_off[vb + lo + 1] - t.node0);
+    t.Lb = t.L > 0 ? t.L : 1;
+    const int64_t k = tile - vtile[lo];
+    t.r0 = vrow[lo] + k * kRowSortTile;
+    t.r1 = min(t.r0 + kRowSortTile, vrow[lo + 1]);
+    t.tab = vtab[lo] + k * t.Lb;
+    int b = 0, bh = nb; // largest block b with blk_row_off[b] <= r0
+    while (bh - b > 1) {
+      const int mid = (b + bh) >> 1;
+      if (blk_row_off[mid] <= t.r0) b = mid; else bh = mid;
+    }
+    t.b0 = b;
+    s_rt = t;
+  }
+  __syncthreads();
+  rt = s_rt;
+}
+
+// Histogram of the tile's local line ids into its table row; index validation and clamping as expand_rows_kernel.
+__global__ void __launch_bounds__(kRowSortThreads)
+row_count_kernel(const int32_t *__restrict__ pairs, const int64_t *__restrict__ blk_row_off,
+                 const int32_t *__restrict__ blk_ng, const int64_t *__restrict__ blk_pair_off, int nb,
+                 const int64_t *__restrict__ line_off, int vb, const int64_t *__restrict__ vrow,
+                 const int32_t *__restrict__ vtile, const int64_t *__restrict__ vtab, int i_lo, int i_hi, int tile0,
+                 uint32_t *__restrict__ tab, int *err) {
+  extern __shared__ uint32_t hist[];
+  RowTile rt;
+  row_tile_of(tile0 + blockIdx.x, blk_row_off, nb, line_off, vb, vrow, vtile, vtab, i_lo, i_hi, rt);
+  for (int b = threadIdx.x; b < rt.Lb; b += kRowSortThreads) hist[b] = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  int b = rt.b0;
+  for (int64_t rr = rt.r0; rr < rt.r1; rr += kRowSortThreads) {
+    const int64_t r = rr + threadIdx.x;
+    int bin = -1;
+    if (r < rt.r1) {
+      while (blk_row_off[b + 1] <= r) ++b;
+      const int2 pr = reinterpret_cast<const int2 *>(pairs)[blk_pair_off[b] + (r - blk_row_off[b])];
+      const int nv = blk_ng[b];
+      const int64_t nl_ng = line_off[nv + 1] - line_off[nv];
+      bin = pr.x;
+      if (bin < 0 || bin >= rt.L) { *err = 1; bin = 0; }
+      if (pr.y < 0 || pr.y >= nl_ng) *err = 2;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, bin);
+    if (bin >= 0 && (__ffs(peers) - 1) == lane) atomicAdd(&hist[bin], (uint32_t)__popc(peers));
+  }
+  __syncthreads();
+  for (int k = threadIdx.x; k < rt.Lb; k += kRowSortThreads) tab[rt.tab + k] = hist[k];
+}
+
+// Per view (one CTA): exclusive prefix of every line's counts over the view's tiles, in place, and the node row
+// offsets of the view's lines (a block scan of the line totals from the view's first row). Largest node -> max_rows.
+__global__ void __launch_bounds__(kRowSortThreads)
+row_scan_kernel(const int64_t *__restrict__ line_off, int vb, int i_lo, const int64_t *__restrict__ vrow,
+                const int32_t *__restrict__ vtile, const int64_t *__restrict__ vtab, uint32_t *__restrict__ tab,
+                uint32_t *__restrict__ node_row_off, unsigned int *max_rows) {
+  typedef cub::BlockScan<uint32_t, kRowSortThreads> Scan;
+  __shared__ typename Scan::TempStorage ts;
+  const int i = i_lo + blockIdx.x;
+  const int64_t node0 = line_off[vb + i], L = line_off[vb + i + 1] - node0;
+  // the group's last node boundary (also the first row of the next view: the same value as any writer of it)
+  if (threadIdx.x == 0 && blockIdx.x == gridDim.x - 1) node_row_off[node0 + L] = (uint32_t)vrow[i + 1];
+  if (L > kRowSortMaxLines) return; // radix-sort fallback view
+  const int nt = vtile[i + 1] - vtile[i];
+  uint32_t *tb = tab + vtab[i];
+  uint32_t run = (uint32_t)vrow[i], mx = 0;
+  for (int64_t l0 = 0; l0 < L; l0 += kRowSortThreads) {
+    const int64_t l = l0 + threadIdx.x;
+    uint32_t tot = 0;
+    if (l < L) {
+#pragma unroll 4
+      for (int t = 0; t < nt; ++t) {
+        const uint32_t c = tb[(int64_t)t * L + l];
+        tb[(int64_t)t * L + l] = tot;
+        tot += c;
+      }
+    }
+    mx = max(mx, tot);
+    uint32_t ex, agg;
+    Scan(ts).ExclusiveSum(tot, ex, agg);
+    if (l < L) node_row_off[node0 + l] = run + ex;
+    run += agg;
+    __syncthreads();
+  }
+  mx = __reduce_max_sync(0xffffffffu, mx);
+  if ((threadIdx.x & 31) == 0 && mx) atomicMax(max_rows, mx);
+}
+
+// Rows of the tile to their slots. Warp w owns rows [r0 + w * kRowSortSlice, ...) of the tile: it counts its slice per
+// line, the counts of the warps are combined in warp order on top of the tile's slot per line, and the warp then walks
+// its slice again in row order, ranking equal lines inside each 32-row step with __match_any_sync.
+__global__ void __launch_bounds__(kRowSortThreads)
+row_scatter_kernel(const int32_t *__restrict__ pairs, const int64_t *__restrict__ blk_row_off,
+                   const int32_t *__restrict__ blk_ng, const int64_t *__restrict__ blk_pair_off, int nb,
+                   const int64_t *__restrict__ line_off, int vb, const int64_t *__restrict__ vrow,
+                   const int32_t *__restrict__ vtile, const int64_t *__restrict__ vtab, int i_lo, int i_hi, int tile0,
+                   const uint32_t *__restrict__ tab, const uint32_t *__restrict__ node_row_off,
+                   uint32_t *__restrict__ key, uint32_t *__restrict__ val) {
+  extern __shared__ uint32_t ctr[]; // [warp][Lb]: the warp's count per line, then its next slot per line
+  RowTile rt;
+  row_tile_of(tile0 + blockIdx.x, blk_row_off, nb, line_off, vb, vrow, vtile, vtab, i_lo, i_hi, rt);
+  for (int k = threadIdx.x; k < kRowSortWarps * rt.Lb; k += kRowSortThreads) ctr[k] = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  uint32_t *wc = ctr + w * rt.Lb;
+  const int64_t ws = rt.r0 + (int64_t)w * kRowSortSlice, we = min(ws + kRowSortSlice, rt.r1);
+  int b = rt.b0;
+  for (int64_t rr = ws; rr < we; rr += 32) {
+    const int64_t r = rr + lane;
+    int bin = -1;
+    if (r < we) {
+      while (blk_row_off[b + 1] <= r) ++b;
+      bin = reinterpret_cast<const int2 *>(pairs)[blk_pair_off[b] + (r - blk_row_off[b])].x;
+      if (bin < 0 || bin >= rt.L) bin = 0;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, bin);
+    if (bin >= 0 && (__ffs(peers) - 1) == lane) wc[bin] += (uint32_t)__popc(peers);
+    __syncwarp();
+  }
+  __syncthreads();
+  for (int k = threadIdx.x; k < rt.Lb; k += kRowSortThreads) {
+    // (a view without lines only has out-of-range rows, clamped to line 0: keep them inside the view's rows)
+    uint32_t base = (k < rt.L ? node_row_off[rt.node0 + k] : (uint32_t)vrow[rt.i]) + (rt.L > 0 ? tab[rt.tab + k] : 0u);
+    for (int ww = 0; ww < kRowSortWarps; ++ww) {
+      const uint32_t c = ctr[ww * rt.Lb + k];
+      ctr[ww * rt.Lb + k] = base;
+      base += c;
+    }
+  }
+  __syncthreads();
+  b = rt.b0;
+  const unsigned lt = (1u << lane) - 1u;
+  for (int64_t rr = ws; rr < we; rr += 32) {
+    const int64_t r = rr + lane;
+    int bin = -1, nv = 0, ngl = 0;
+    if (r < we) {
+      while (blk_row_off[b + 1] <= r) ++b;
+      const int2 pr = reinterpret_cast<const int2 *>(pairs)[blk_pair_off[b] + (r - blk_row_off[b])];
+      nv = blk_ng[b];
+      const int64_t nl_ng = line_off[nv + 1] - line_off[nv];
+      bin = pr.x;
+      ngl = pr.y;
+      if (bin < 0 || bin >= rt.L) bin = 0;
+      if (ngl < 0 || ngl >= nl_ng) ngl = 0;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, bin);
+    const uint32_t pos = bin >= 0 ? wc[bin] + (uint32_t)__popc(peers & lt) : 0u;
+    __syncwarp();
+    if (bin >= 0 && (__ffs(peers) - 1) == lane) wc[bin] += (uint32_t)__popc(peers);
+    __syncwarp();
+    if (bin >= 0) {
+      key[pos] = (uint32_t)(rt.node0 + bin);
+      val[pos] = ((uint32_t)nv << 16) | (uint32_t)ngl;
+    }
+  }
+}
+
+size_t row_scatter_smem_bytes(int max_lines) { return (size_t)kRowSortWarps * 4 * (size_t)std::max(max_lines, 1); }
+
+void launch_row_views(const int64_t *d_blk_row_off, const int32_t *d_blk_src_view, int n_blocks,
+                      const int64_t *d_line_off, int vb, int n_views, int64_t *d_vrow, int32_t *d_vtile, int64_t *d_vtab,
+                      cudaStream_t s) {
+  row_views_kernel<<<1, kRowSortThreads, 0, s>>>(d_blk_row_off, d_blk_src_view, n_blocks, d_line_off, vb, n_views,
+                                                  d_vrow, d_vtile, d_vtab);
+}
+
+cudaError_t launch_row_sort(const int32_t *d_pairs, const int64_t *d_blk_row_off, const int32_t *d_blk_ng_view,
+                            const int64_t *d_blk_pair_off, int n_blocks, const int64_t *d_line_off, int vb,
+                            const int64_t *d_vrow, const int32_t *d_vtile, const int64_t *d_vtab, int i_lo, int i_hi,
+                            int tile0, int n_tiles, int max_lines, uint32_t *d_tab, uint32_t *d_node_row_off,
+                            unsigned int *d_max_rows, uint32_t *d_key, uint32_t *d_val, int *d_err, cudaStream_t s) {
+  if (i_hi <= i_lo) return cudaSuccess;
+  if (n_tiles > 0)
+    row_count_kernel<<<n_tiles, kRowSortThreads, 4 * std::max(max_lines, 1), s>>>(
+        d_pairs, d_blk_row_off, d_blk_ng_view, d_blk_pair_off, n_blocks, d_line_off, vb, d_vrow, d_vtile, d_vtab, i_lo,
+        i_hi, tile0, d_tab, d_err);
+  row_scan_kernel<<<i_hi - i_lo, kRowSortThreads, 0, s>>>(d_line_off, vb, i_lo, d_vrow, d_vtile, d_vtab, d_tab,
+                                                          d_node_row_off, d_max_rows);
+  if (n_tiles > 0) {
+    const size_t smem = row_scatter_smem_bytes(max_lines);
+    if (smem > 48 * 1024) {
+      const cudaError_t e = cudaFuncSetAttribute(row_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+      if (e != cudaSuccess) return e;
+    }
+    row_scatter_kernel<<<n_tiles, kRowSortThreads, smem, s>>>(d_pairs, d_blk_row_off, d_blk_ng_view, d_blk_pair_off,
+                                                              n_blocks, d_line_off, vb, d_vrow, d_vtile, d_vtab, i_lo,
+                                                              i_hi, tile0, d_tab, d_node_row_off, d_key, d_val);
+  }
+  return cudaGetLastError();
 }
 
 // valid_edges_ (global_line_triangulator.cc:130-142) in compact, node-major, candidate-ordered form.

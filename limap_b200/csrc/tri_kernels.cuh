@@ -103,6 +103,19 @@ void launch_expand_exhaustive(const int64_t *d_blk_row_off, const int32_t *d_blk
                               int64_t n_rows, uint32_t *d_key, uint32_t *d_val, cudaStream_t s);
 void launch_node_offsets(const uint32_t *d_sorted_key, int64_t n_rows, int64_t row_base, int64_t node_lo,
                          int64_t node_hi, uint32_t *d_node_row_off, unsigned int *d_max_rows, cudaStream_t s);
+// Node-major rows by a per-view stable counting sort (non-exhaustive matches). A view with more lines than
+// kRowSortMaxLines keeps the radix-sort path; kRowSortTile rows of a view form one tile (one CTA).
+static constexpr int kRowSortMaxLines = 4096;
+static constexpr int kRowSortTile = 8192;
+size_t row_scatter_smem_bytes(int max_lines);
+void launch_row_views(const int64_t *d_blk_row_off, const int32_t *d_blk_src_view, int n_blocks,
+                      const int64_t *d_line_off, int vb, int n_views, int64_t *d_vrow, int32_t *d_vtile, int64_t *d_vtab,
+                      cudaStream_t s);
+cudaError_t launch_row_sort(const int32_t *d_pairs, const int64_t *d_blk_row_off, const int32_t *d_blk_ng_view,
+                            const int64_t *d_blk_pair_off, int n_blocks, const int64_t *d_line_off, int vb,
+                            const int64_t *d_vrow, const int32_t *d_vtile, const int64_t *d_vtab, int i_lo, int i_hi,
+                            int tile0, int n_tiles, int max_lines, uint32_t *d_tab, uint32_t *d_node_row_off,
+                            unsigned int *d_max_rows, uint32_t *d_key, uint32_t *d_val, int *d_err, cudaStream_t s);
 void launch_extract_nvalid(const NodeRecord *nodes, int64_t node_begin, int64_t n, uint32_t *out, cudaStream_t s);
 void launch_compact_edges_only(const uint8_t *row_state, const uint32_t *row_ng, const uint32_t *node_row_off,
                                const uint32_t *edge_off, int64_t node_begin, int64_t n, int ns, uint32_t *edge_ng,
